@@ -2,7 +2,7 @@
 """bench.py — SVG tokens/sec of the im2svg hot path (BASELINE.json metric), one JSON line on rank 0.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--max-new-tokens 4096] [--batch-per-gpu 1] [--no-cpu-baseline]
+                    [--max-new-tokens 4096] [--batch-per-gpu 1] [--no-cpu-baseline] [--dump-outputs DIR]
 
 A "step" is one full `generate_im2svg` pass over one batch of synthetic 224x224 images with
 random-init StarVector-1B weights: ViT -> adapter -> decoder prefill -> `max_new_tokens` greedy
@@ -13,6 +13,8 @@ decode steps (EOS/stop disabled so the length is deterministic, SURVEY.md §8d).
   cpu_baseline : the CPU oracle (HF generate on the host cores) on a bounded sample, rank 0, N=1
 `--impl reference` times that CPU path as the reference arm (the reference is pure Python and has
 no GPU-independent build; its own decoder is the installed `transformers` class).
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float32), so that
+two builds can be compared output for output: the inputs are seeded, identical from run to run.
 """
 from __future__ import annotations
 
@@ -106,13 +108,12 @@ def cpu_generate_seconds(o, d, img, n_new):
     return time.perf_counter() - t0, ids[0, len(PROMPT_IDS):].tolist()
 
 
-def cpu_reference_run(threads: int, steps: int = 1, warmup: int = 1, n_new: int = CONFIG1_NEW, budget_s: float = 150.0,
+def cpu_reference_run(threads: int, steps: int = 1, warmup: int = 1, n_new: int = CONFIG1_NEW,
                       target_new: int = 4096, try_bf16: bool = True):
     """BASELINE.json configs[0] literally: the CPU oracle (reference ViT/adapter modules + the installed transformers
     `GPTBigCodeForCausalLM.generate`, oracle/pipeline.py) generates `n_new` = 256 greedy tokens for one image in fp32;
-    every timed step is one whole such call (ViT + adapter + 259-token prefill + 256 decode steps).  Steps stop early when
-    `budget_s` is spent (the count actually run is reported).  A short generation (8 tokens) separates the fixed prefix
-    cost from the per-token cost, so that the projection to the GPU arm's `target_new`-token workload can be stated next
+    every timed step is one whole such call (ViT + adapter + 259-token prefill + 256 decode steps), `steps` of them.
+    A short generation (8 tokens) separates the fixed prefix cost from the per-token cost, so that the projection to the GPU arm's `target_new`-token workload can be stated next
     to the measured number.  bf16 (BASELINE.md §3 asks for both) is attempted on 8 tokens first and only run in full when
     the host executes bf16 matmuls natively (AMX); otherwise the reason is recorded."""
     torch.set_num_threads(threads)
@@ -121,12 +122,9 @@ def cpu_reference_run(threads: int, steps: int = 1, warmup: int = 1, n_new: int 
     for _ in range(max(1, warmup)):                      # warm-up: allocator, oneDNN primitive caches (short runs)
         t_short, _ = cpu_generate_seconds(o, d, img, 8)
     times, ids = [], None
-    t_begin = time.perf_counter()
-    for _ in range(max(1, steps)):
+    for _ in range(steps):
         t, ids = cpu_generate_seconds(o, d, img, n_new)
         times.append(t)
-        if time.perf_counter() - t_begin > budget_s:
-            break
     sec = sum(times) / len(times)
     per_tok = max(sec - t_short, 1e-9) / (n_new - 8)
     prefix = max(t_short - 8 * per_tok, 0.0)
@@ -180,6 +178,8 @@ def run_reference(args):
         return
     threads = min(os.cpu_count() or 1, CPU_THREADS_CAP)
     r = cpu_reference_run(threads, steps=args.steps, warmup=min(args.warmup, 2), target_new=args.max_new_tokens)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ids": torch.tensor([r["ids"]])})
     v = r["tokens_per_s"]
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": "tokens/s", "n_gpus": args.gpus, "steps": r["steps_run"],
@@ -200,6 +200,22 @@ def ids_digest(ids: torch.Tensor) -> str:
     import hashlib
 
     return hashlib.sha256(ids.detach().to("cpu", torch.int32).contiguous().numpy().tobytes()).hexdigest()[:16]
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """arrays: name -> tensor, written as out_dir/<name>.npy in float32 (token ids < 2**24 are exact)."""
+    import numpy as np
+
+    host = {k: v.detach().to("cpu", torch.float32).contiguous().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench: --dump-outputs would write {total} bytes, over the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def measure(model: str, B: int, n_new: int, steps: int, warmup: int, world: int, rank: int, local: int, sampling: bool = False,
@@ -292,7 +308,7 @@ def measure(model: str, B: int, n_new: int, steps: int, warmup: int, world: int,
         total_ms = float(ms_t.item())
     launches = eng.launch_count() - launches0
     digests = [ids_digest(x) for x in passes]                 # after the timed region: what did the timed passes produce?
-    first_ids = passes[0].detach().cpu()
+    first_ids, last_ids = passes[0].detach().cpu(), passes[-1].detach().cpu()
     del passes
 
     def prefill_only():
@@ -323,7 +339,7 @@ def measure(model: str, B: int, n_new: int, steps: int, warmup: int, world: int,
     return {
         "dims": d, "gb": gb, "t0": t0, "value": value, "e2e_value": e2e_value, "ms_per_step": ms_per_step, "prefill_ms_per_image": pf_ms / 5 / B,
         "step_ms": step_ms, "launches": int(launches), "engine": desc, "clocks": clocks.summary(), "achieved": achieved, "peak": peak,
-        "peak_src": peak_src, "bytes_per_step": int(bytes_per_step), "first_ids": first_ids,
+        "peak_src": peak_src, "bytes_per_step": int(bytes_per_step), "first_ids": first_ids, "last_ids": last_ids,
         "ids": {"sha256_16_per_pass": digests, "host_path": digests_host,
                 "identical_across_passes_and_paths": same if not sampling else None},
     }
@@ -378,7 +394,11 @@ def main():
     ap.add_argument("--model", default="1b", choices=["1b", "8b"],
                     help="1b = StarVector-1B (headline, configs[1]); 8b = StarVector-8B family dims (SigLIP + StarCoder2)")
     ap.add_argument("--sampling", action="store_true", help="temperature 0.8 / top_p 0.9 sampling instead of greedy (BASELINE configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the generated ids of the last timed step as DIR/ids.npy (float32) after the timed steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         return run_reference(args)
@@ -402,6 +422,8 @@ def main():
     d = m["dims"]
     if m["ids"]["identical_across_passes_and_paths"] is False:
         raise SystemExit(f"bench: greedy passes produced different ids {m['ids']}: the timed work is not deterministic - refusing to report")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"ids": m["last_ids"]})
     workload = WORKLOAD if args.model == "1b" else WORKLOAD.replace("StarVector-1B", "StarVector-8B (SigLIP-L/16-384 + StarCoder2-7B dims)").replace("224x224", "384x384")
     if args.sampling:
         workload = workload.replace("greedy", "sampling T=0.8 top_p=0.9")

@@ -212,3 +212,18 @@ def test_v2_tokenizer_preparation(tmp_path):
         assert len(tok.encode(t)) == 1
     syn = load_tokenizer(None, 500, v2=True)
     assert isinstance(syn, SyntheticTokenizer) and syn.padding_side == "left" and syn.pad_token_id == 495
+
+
+def test_bench_dump_outputs_writes_float32_arrays(tmp_path):
+    """bench.py --dump-outputs: every array as <name>.npy in float32 with the values unchanged; over 64 MB in all is refused."""
+    import numpy as np
+
+    import bench
+
+    ids = torch.tensor([[44, 49151, 0, 16777215]], dtype=torch.int32)
+    bench.dump_outputs(str(tmp_path / "out"), {"ids": ids})
+    got = np.load(tmp_path / "out" / "ids.npy")
+    assert got.dtype == np.float32 and got.shape == (1, 4) and np.array_equal(got, ids.numpy())
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "big"), {"ids": torch.zeros(bench.DUMP_LIMIT_BYTES // 4 + 1, dtype=torch.int32)})
+    assert not (tmp_path / "big").exists()

@@ -1,18 +1,17 @@
 """Pin the CPU oracle (oracle/) against fixtures produced by the reference's own modules.
 
-tests/golden/tiny_v1_*.pt were written by `python -m oracle.make_golden`, which imports
-VisionTransformer / LayerNorm / Adapter from /root/reference and drives the installed
-transformers GPTBigCode through generate().  Here (no /root/reference needed) the oracle
-restatement must reproduce them; when /root/reference is mounted, it is additionally checked
-bit-for-bit against the live reference modules.
+tests/golden/tiny_v1_*.pt were written by `python -m oracle.make_golden` and
+`python -m oracle.make_golden_reference`, which run VisionTransformer / LayerNorm / Adapter of the
+reference checkout and drive the installed transformers GPTBigCode through generate().  The oracle
+restatement must reproduce them: within 2 bf16 ulps of the fixtures taken with oneDNN on, and bit for
+bit with oneDNN off on both sides.
 """
 import os
 
 import pytest
 import torch
 
-from oracle import ref_shim
-from oracle.pipeline import ADP, LNV, VIS, OracleStarVector
+from oracle.pipeline import OracleStarVector
 from starvector_b200.config import ModelDims
 from starvector_b200.weights import synthetic_images, synthetic_state_dict
 
@@ -75,23 +74,17 @@ def test_row0_stop_stops_whole_batch(golden_dir):
     assert out.shape[1] == first + 3 and torch.equal(out, base[:, : first + 3])
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not mounted (GPU box)")
 @pytest.mark.parametrize("norm", ["layer_norm", "batch_norm"])
-def test_restatement_bit_exact_vs_live_reference(golden_dir, norm):
+def test_restatement_bit_exact_vs_reference_outputs(golden_dir, norm):
+    """Same operations in the same order as the reference modules: equal bits.  oneDNN stays off on both sides because its AMX
+    and AVX kernels round bf16 matmuls differently (oracle/make_golden_reference.py)."""
+    torch.set_num_threads(1)
     g, d, sd, img = _load(golden_dir, norm)
-    VT, LN, AD = ref_shim.load()
-    vt = VT(d.image_size, d.patch_size, d.vit_width, d.vit_layers, d.vit_heads, False)
-    vt.load_state_dict({k[len(VIS):]: v for k, v in sd.items() if k.startswith(VIS)})
-    ln = LN(d.vit_width)
-    ln.load_state_dict({k[len(LNV):]: v for k, v in sd.items() if k.startswith(LNV)})
-    ad = AD(d.vit_width, d.hidden, adapter_norm=norm, query_length=d.query_length)
-    ad.load_state_dict({k[len(ADP):]: v for k, v in sd.items() if k.startswith(ADP)}, strict=False)
-    vt, ln, ad = vt.to(torch.bfloat16).eval(), ln.to(torch.bfloat16).eval(), ad.to(torch.bfloat16).eval()
+    ref = torch.load(os.path.join(golden_dir, "tiny_v1_reference_vision.pt"), weights_only=False)[norm]
     o = OracleStarVector(d, sd, dtype=torch.bfloat16, pad_token_id=d.vocab - 4)
-    with torch.no_grad():
-        ref_v = ln(vt(img))
-        assert torch.equal(ref_v, o.image_encoder(img))
-        assert torch.equal(ad(ref_v), o.image_projection(ref_v))
+    with torch.no_grad(), torch.backends.mkldnn.flags(enabled=False):
+        assert torch.equal(o.image_encoder(img), ref["vit_out"])
+        assert torch.equal(o.image_projection(ref["vit_out"]), ref["adapter_out"])
 
 
 def test_v2_oracle_matches_fixture(golden_dir):

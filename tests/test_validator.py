@@ -1,6 +1,7 @@
 """Validator backend (starvector_b200/validator.py): the reference's registry accepts it and `generate_svg` follows
 starvector_hf_validator.py:77-88.  The model is a recording stand-in: no GPU is needed for the contract."""
-import importlib.util
+import abc
+import json
 import os
 import sys
 import types
@@ -9,8 +10,6 @@ import pytest
 import torch
 
 from starvector_b200 import validator as V
-
-REF = "/root/reference/starvector/validation/svg_validator_base.py"
 
 
 class _FakeCore:
@@ -30,29 +29,30 @@ class _FakeModel:
         self.device = torch.device("cpu")
 
 
-def _load_reference_base():
-    """svg_validator_base.py imported from its file with stand-ins for what this container lacks (omegaconf, svgpathtools, the
-    metrics package, cairosvg-backed data utils): the registry, the decorator and the ABC are the reference's own code."""
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        sys.modules[name] = m
-        return m
+def _load_reference_base(golden_dir):
+    """A stand-in for the reference's svg_validator_base module, built from what oracle/make_golden_reference.py recorded of
+    it (tests/golden/validator_registry.json): its import path, the abstract methods of `SVGValidator` and the class attribute
+    `register_validator` files a class under."""
+    with open(os.path.join(golden_dir, "validator_registry.json")) as f:
+        spec = json.load(f)
+    pkg, _, leaf = spec["module"].rpartition(".")
+    saved = {k: sys.modules.get(k) for k in ("starvector", pkg, spec["module"])}
+    for n in ("starvector", pkg):
+        m = types.ModuleType(n)
+        m.__path__ = []
+        sys.modules[n] = m
+    mod = types.ModuleType(spec["module"])
+    mod.validator_registry = {}
+    mod.SVGValidator = abc.ABCMeta("SVGValidator", (abc.ABC,), {n: abc.abstractmethod(lambda self, *a, **k: None)
+                                                                for n in spec["abstract_methods"]})
 
-    saved = {k: sys.modules.get(k) for k in ("omegaconf", "svgpathtools", "starvector", "starvector.validation", "starvector.metrics",
-                                             "starvector.metrics.metrics", "starvector.data", "starvector.data.util",
-                                             "starvector.validation.svg_validator_base")}
-    stub("omegaconf", OmegaConf=type("OmegaConf", (), {"save": staticmethod(lambda **k: None), "load": staticmethod(lambda p: {"metrics": {}})}))
-    stub("svgpathtools", svgstr2paths=lambda s: None)
-    for n in ("starvector", "starvector.validation", "starvector.metrics", "starvector.data"):
-        stub(n).__path__ = []
-    stub("starvector.metrics.metrics", SVGMetrics=lambda cfg: None)
-    stub("starvector.data.util", rasterize_svg=lambda *a, **k: None, clean_svg=lambda s: s, use_placeholder=lambda: "<svg></svg>")
-    spec = importlib.util.spec_from_file_location("starvector.validation.svg_validator_base", REF)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[spec.name] = mod
-    spec.loader.exec_module(mod)
-    sys.modules["starvector.validation"].svg_validator_base = mod
+    def register_validator(cls):
+        mod.validator_registry[getattr(cls, spec["registry_key"])] = cls
+        return cls
+
+    mod.register_validator = register_validator
+    sys.modules[spec["module"]] = mod
+    setattr(sys.modules[pkg], leaf, mod)
     return mod, saved
 
 
@@ -76,9 +76,8 @@ def test_generate_svg_follows_the_hf_backend():
         v.generate_svg({"image": torch.zeros(1, 3, 8, 8)}, cfg)
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="/root/reference is not mounted")
-def test_registers_with_the_reference_registry():
-    mod, saved = _load_reference_base()
+def test_registers_with_the_reference_registry(golden_dir):
+    mod, saved = _load_reference_base(golden_dir)
     try:
         cls = V.register()
         assert mod.validator_registry[V.ENGINE_NAME] is cls and issubclass(cls, mod.SVGValidator)
