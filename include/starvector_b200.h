@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SV_ABI_VERSION 4
+#define SV_ABI_VERSION 5
 #if defined(__GNUC__)
 #define SV_API __attribute__((visibility("default")))
 #else
@@ -235,6 +235,40 @@ SV_API int sv_op_linear(int32_t impl, const void* x, const void* w, const void* 
 SV_API int sv_op_attention_vit(const void* qkv, void* out, int32_t batch, int32_t seq, int32_t heads, void* stream);
 /* Causal multi-query attention over packed qkv [B*T, heads*D + 2*D] (D=128) -> out [B*T, heads*D]. */
 SV_API int sv_op_attention_mqa(const void* qkv, void* out, int32_t batch, int32_t seq, int32_t heads, void* stream);
+/* Causal grouped-query attention of the decoder prefill over packed qkv [B*T, (n_head + 2*n_kv)*D] (D=128)
+ * -> out [B*T, n_head*D]; window > 0 restricts token t to keys (t - window, t] (StarCoder2 sliding window). */
+SV_API int sv_op_attention_prefill(const void* qkv, void* out, int32_t batch, int32_t seq, int32_t n_head, int32_t n_kv,
+                                   int32_t window, void* stream);
+
+/* The decode-step kernels one at a time.  Each call validates its arguments before any launch (SV_ERR_INVALID),
+ * allocates its own scratch (generation state, partial buffers, tiled weight copy) and synchronises `stream`. */
+enum { SV_ATTN_DECODE_CLUSTER = 0, SV_ATTN_DECODE_SPLIT = 1 };
+/* One decode token per row: q [B, n_head*D] against K [B][n_kv][tcap][D] and V^T [B][n_kv][D][tcap] -> out [B, n_head*D].
+ * Keys [max(0, nkeys - window), nkeys) take part (window 0 = all); 1 <= nkeys <= tcap, tcap % 32 == 0, B <= 8, group <= 16.
+ * nparts forces the cluster size (1..8) or the split count (1..128); 0 = what the engine picks for nkeys. */
+SV_API int sv_op_attention_decode(int32_t impl, const void* q, const void* kcache, const void* vtcache, void* out,
+                                  int32_t batch, int32_t n_head, int32_t n_kv, int32_t tcap, int32_t nkeys, int32_t window,
+                                  int32_t nparts, void* stream);
+enum { SV_GEMV_EPI_PLAIN = 0, SV_GEMV_EPI_QKV = 1, SV_GEMV_EPI_LMHEAD = 2 };
+/* One weight-ring decode GEMV: y[B,N] = epilogue(LayerNorm?(x)[B,K] . w[N,K]^T), B <= 8, K % 32 == 0; LayerNorm when
+ * ln_w / ln_b are given; bias, residual (may alias y) optional.  Epilogues: SV_GEMV_EPI_QKV also appends the K row and the
+ * V^T column at `pos` of the caches (N == (n_head + 2*n_kv)*128, pos < tcap); SV_GEMV_EPI_LMHEAD also writes per-tile
+ * argmax partials amax_val float / amax_idx int32 [tile][8] (capacity in tiles).  tiled = 1 streams a slab-tiled copy of
+ * w made inside the call.  *ntiles_out (host, optional) = the number of partial tiles. */
+SV_API int sv_op_gemv_ring(const void* x, const void* w, const void* bias, const void* residual, const void* ln_w,
+                           const void* ln_b, void* y, int32_t batch, int32_t N, int32_t K, int32_t act, float ln_eps,
+                           int32_t epi, int32_t tiled, void* kcache, void* vtcache, int32_t n_head, int32_t n_kv,
+                           int32_t tcap, int32_t pos, float* amax_val, int32_t* amax_idx, int32_t amax_capacity,
+                           int32_t* ntiles_out, void* stream);
+enum { SV_SELECT_GREEDY = 0, SV_SELECT_FUSED = 1, SV_SELECT_FUSED_PARTIALS = 2, SV_SELECT_SAMPLE = 3 };
+/* Token selection of one step from bf16 logits [B,V] and a seen bitmap uint8 [B,V] (host or device; not modified) at
+ * generation step `step` with `cur_len` tokens in the cache -> tokens int32 [B] (host or device).  The fused kernels also
+ * write x_out [B,h] = wte[token] + wpe[min(cur_len + 1, n_positions - 1)] (wpe may be NULL); SV_SELECT_FUSED_PARTIALS
+ * reduces lm_head argmax partials [ntiles][8] instead of the logits. */
+SV_API int sv_op_select(int32_t mode, const void* logits, const uint8_t* seen, const sv_gen_params* p, int32_t batch,
+                        int32_t vocab, int32_t step, int32_t cur_len, const float* amax_val, const int32_t* amax_idx,
+                        int32_t ntiles, const void* wte, const void* wpe, int32_t h, int32_t n_positions, void* x_out,
+                        int32_t* tokens, void* stream);
 
 /* ---- image preprocessing (SURVEY.md §8f-2) ------------------------------------------------ */
 /* Replaces `ImageTrainProcessor.__call__` (reference starvector/data/util.py:40-66: RGBA pasted on white, pad to

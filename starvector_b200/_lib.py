@@ -16,7 +16,10 @@ SV_OK, SV_ERR_INVALID, SV_ERR_CUDA, SV_ERR_UNSUPPORTED, SV_ERR_STATE = 0, -1, -2
 SV_DTYPE_BF16, SV_DTYPE_F32, SV_DTYPE_F16 = 0, 1, 2
 SV_ACT_NONE, SV_ACT_QUICKGELU, SV_ACT_GELU_TANH, SV_ACT_SILU = 0, 1, 2, 3
 SV_LINEAR_AUTO, SV_LINEAR_ROWGROUP, SV_LINEAR_TCGEN05 = 0, 1, 2
-ABI_VERSION = 4
+SV_ATTN_DECODE_CLUSTER, SV_ATTN_DECODE_SPLIT = 0, 1
+SV_GEMV_EPI_PLAIN, SV_GEMV_EPI_QKV, SV_GEMV_EPI_LMHEAD = 0, 1, 2
+SV_SELECT_GREEDY, SV_SELECT_FUSED, SV_SELECT_FUSED_PARTIALS, SV_SELECT_SAMPLE = 0, 1, 2, 3
+ABI_VERSION = 5
 SV_ALPHA_WHITE, SV_ALPHA_DROP = 0, 1
 
 
@@ -93,6 +96,11 @@ SIGNATURES = {
     "sv_op_linear": (C.c_int, [_I, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "sv_op_attention_vit": (C.c_int, [_P, _P, _I, _I, _I, _P]),
     "sv_op_attention_mqa": (C.c_int, [_P, _P, _I, _I, _I, _P]),
+    "sv_op_attention_prefill": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _P]),
+    "sv_op_attention_decode": (C.c_int, [_I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "sv_op_gemv_ring": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _I, _P, _P, _I, _I, _I, _I, _P, _P, _I,
+                                  C.POINTER(_I), _P]),
+    "sv_op_select": (C.c_int, [_I, _P, _P, C.POINTER(GenParams), _I, _I, _I, _I, _P, _P, _I, _P, _P, _I, _I, _P, _P, _P]),
     "sv_preproc_create": (C.c_int, [C.POINTER(PreprocDesc), C.c_int, C.POINTER(_P)]),
     "sv_preproc_destroy": (None, [_P]),
     "sv_preproc_last_error": (C.c_char_p, [_P]),

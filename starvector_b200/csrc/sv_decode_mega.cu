@@ -38,8 +38,8 @@ struct Ctx {
 };
 
 // ---- consumer: one GEMV phase  Y[B,N] = epi( LN?(X)[B,K] . W[N,K]^T )
-// LN_BIGK compiles in the LayerNorm path for K > 2048 (v2); v1 kernels are instantiated without it so their register
-// allocation is untouched.
+// LN_BIGK compiles in the LayerNorm path for phases of more than two slabs (K > 2048, or a K only a narrow slab divides);
+// the other kernels are instantiated without it so their register allocation is untouched.
 template <bool HAS_LN, int EPI, bool LN_BIGK = false>
 SV_DEVINL void gemv_phase(const Ctx& cx, Ring& r, const bf16* __restrict__ X, const bf16* __restrict__ bias,
                           const bf16* res, bf16* Y, int N, int K, int act, const bf16* __restrict__ ln_w,
@@ -441,6 +441,8 @@ cudaError_t gemv_ring_init() {   // set the shared-memory opt-in outside of any 
   SV_RING_ATTR(true, mega::EPI_QKV) SV_RING_ATTR(true, mega::EPI_PLAIN) SV_RING_ATTR(true, mega::EPI_LMHEAD)
   SV_RING_ATTR(false, mega::EPI_PLAIN)
 #undef SV_RING_ATTR
+  e = cudaFuncSetAttribute(mega::gemv_ring_kernel<true, mega::EPI_QKV, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mega::SMEM_BYTES);
+  if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(mega::gemv_ring_kernel<true, mega::EPI_PLAIN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mega::SMEM_BYTES);
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(mega::gemv_ring_kernel<true, mega::EPI_LMHEAD, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mega::SMEM_BYTES);
@@ -474,19 +476,24 @@ void launch_gemv_ring(const RingGemvLaunch& g, cudaStream_t st) {
   ra.X = g.X; ra.W = g.W; ra.Wt = g.Wt; ra.bias = g.bias; ra.res = g.res; ra.ln_w = g.ln_w; ra.ln_b = g.ln_b; ra.Y = g.Y;
   ra.N = g.N; ra.K = g.K; ra.act = g.act;
   const int nsm = gemv_ring_ncta();
+  int nstg = 1;
   {   // ring depth: what this CTA will stream, capped so the next kernel's CTA can co-reside (227 KB per SM)
     static int cap = 0;
     if (cap == 0) { const char* c = getenv("SV_RING_SLOTS"); cap = c ? atoi(c) : mega::STAGES; if (cap < 1 || cap > 6) cap = mega::STAGES; }
     const int rows_per_cta = (g.N + nsm - 1) / nsm, tpc = (rows_per_cta + 15) / 16;
     int ks = 32;
     for (int c : {1024, 768, 512, 256, 128, 64}) if (c <= g.K && g.K % c == 0) { ks = c; break; }
-    const int need = tpc * (g.K / ks);
+    nstg = g.K / ks;
+    const int need = tpc * nstg;
     ra.nslots = need < cap ? need : cap;
     if (ra.nslots < 1) ra.nslots = 1;
   }
   const bool ln = g.ln_w != nullptr;
-  if (ln && g.K > 2 * mega::KS_MAX) {       // LayerNorm over K > 2048 (v2): separate instantiations
+  // More than two slabs (every K > 2048, and narrower K that only a small slab divides, e.g. 640 = 5 x 128): the activations
+  // are streamed per slab, and only the LN_BIGK instantiations normalise them there.
+  if (ln && nstg > 2) {
     if (g.epi == mega::EPI_LMHEAD) launch_ring_t<true, mega::EPI_LMHEAD, true>(ra, nsm, g.pdl, st);
+    else if (g.epi == mega::EPI_QKV) launch_ring_t<true, mega::EPI_QKV, true>(ra, nsm, g.pdl, st);
     else launch_ring_t<true, mega::EPI_PLAIN, true>(ra, nsm, g.pdl, st);
     return;
   }

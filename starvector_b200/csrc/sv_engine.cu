@@ -1372,4 +1372,187 @@ int sv_op_attention_mqa(const void* qkv, void* out, int32_t batch, int32_t seq, 
   return r == cudaSuccess ? SV_OK : op_fail("attention_mqa", r);
 }
 
+int sv_op_attention_prefill(const void* qkv, void* out, int32_t batch, int32_t seq, int32_t n_head, int32_t n_kv,
+                            int32_t window, void* stream) {
+  if (!qkv || !out || batch < 1 || seq < 1 || n_kv < 1 || n_head < n_kv || n_head % n_kv || n_head / n_kv > 16 || window < 0)
+    return fail(nullptr, SV_ERR_INVALID, "bad attention_prefill arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = 128, tcap = (seq + 31) / 32 * 32, cols = (n_head + 2 * n_kv) * D;
+  const size_t n = (size_t)batch * n_kv * tcap * D;
+  bf16* kc = nullptr;
+  cudaError_t r = cudaMalloc(reinterpret_cast<void**>(&kc), 2 * n * 2);
+  if (r != cudaSuccess) return op_fail("attention_prefill alloc", r);
+  bf16* vc = kc + n;
+  cudaMemsetAsync(kc, 0, 2 * n * 2, st);
+  launch_kv_scatter((const bf16*)qkv, kc, vc, batch, seq, n_head * D, n_kv, D, tcap, 0, st);
+  launch_attention_heads((const bf16*)qkv, cols, kc, vc, (bf16*)out, batch, seq, n_head, n_kv, D, tcap, window, st);
+  r = cudaStreamSynchronize(st);
+  cudaFree(kc);
+  return r == cudaSuccess ? SV_OK : op_fail("attention_prefill", r);
+}
+
+// Scratch of the decode-step entry points: one allocation, freed on every path out.
+namespace {
+struct OpScratch {
+  void* p = nullptr;
+  ~OpScratch() { if (p) cudaFree(p); }
+};
+GenState op_state(int cur_len, int step) {
+  GenState hs;
+  memset(&hs, 0, sizeof(hs));
+  hs.cur_len = cur_len;
+  hs.step = step;
+  for (int b = 0; b < 8; ++b) hs.unfinished[b] = 1;
+  return hs;
+}
+}  // namespace
+
+int sv_op_attention_decode(int32_t impl, const void* q, const void* kcache, const void* vtcache, void* out, int32_t batch,
+                           int32_t n_head, int32_t n_kv, int32_t tcap, int32_t nkeys, int32_t window, int32_t nparts,
+                           void* stream) {
+  if (!q || !kcache || !vtcache || !out) return fail(nullptr, SV_ERR_INVALID, "attention_decode: null pointer");
+  if (impl != SV_ATTN_DECODE_CLUSTER && impl != SV_ATTN_DECODE_SPLIT) return fail(nullptr, SV_ERR_INVALID, "attention_decode: unknown impl %d", impl);
+  if (batch < 1 || batch > 8) return fail(nullptr, SV_ERR_INVALID, "attention_decode: batch %d not in [1,8]", batch);
+  if (n_kv < 1 || n_head < n_kv || n_head % n_kv || n_head / n_kv > 16)
+    return fail(nullptr, SV_ERR_INVALID, "attention_decode: need n_head %% n_kv == 0 and a group of 1..16");
+  if (tcap < 32 || tcap % 32) return fail(nullptr, SV_ERR_INVALID, "attention_decode: tcap %d must be a positive multiple of 32", tcap);
+  if (nkeys < 1 || nkeys > tcap) return fail(nullptr, SV_ERR_INVALID, "attention_decode: nkeys %d not in [1, tcap=%d]", nkeys, tcap);
+  if (window < 0) return fail(nullptr, SV_ERR_INVALID, "attention_decode: window < 0");
+  const int max_parts = impl == SV_ATTN_DECODE_CLUSTER ? 8 : kMaxSplit;
+  if (nparts < 0 || nparts > max_parts) return fail(nullptr, SV_ERR_INVALID, "attention_decode: %d parts not in [0,%d]", nparts, max_parts);
+  if (nparts == 0)   // the engine's choice for this length
+    nparts = impl == SV_ATTN_DECODE_CLUSTER ? attention_decode_cluster_ncta(nkeys) : std::max(1, std::min(kMaxSplit, (nkeys + 31) / 32));
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = 128;
+  const size_t part_bytes = impl == SV_ATTN_DECODE_SPLIT ? (size_t)batch * n_kv * nparts * (32 + 16 * D) * sizeof(float) : 0;
+  OpScratch s;
+  cudaError_t r = cudaMalloc(&s.p, sizeof(GenState) + part_bytes);
+  if (r != cudaSuccess) return op_fail("attention_decode alloc", r);
+  GenState* state = reinterpret_cast<GenState*>(s.p);
+  const GenState hs = op_state(nkeys - 1, 0);      // the kernels attend over keys [.., cur_len] = the new token's own K/V
+  r = cudaMemcpyAsync(state, &hs, sizeof(hs), cudaMemcpyHostToDevice, st);
+  if (r != cudaSuccess) return op_fail("attention_decode state", r);
+  if (impl == SV_ATTN_DECODE_CLUSTER) {
+    r = attention_decode_cluster_init();
+    if (r == cudaSuccess)
+      r = launch_attention_decode_cluster((const bf16*)q, n_head * D, (const bf16*)kcache, (const bf16*)vtcache, (bf16*)out,
+                                          state, batch, n_head, n_kv, D, tcap, nparts, window, false, st);
+  } else {
+    float* part = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(s.p) + sizeof(GenState));
+    launch_attention_decode((const bf16*)q, n_head * D, (const bf16*)kcache, (const bf16*)vtcache, (bf16*)out, part, state,
+                            batch, n_head, n_kv, D, tcap, nparts, window, st);
+  }
+  if (r == cudaSuccess) r = cudaGetLastError();
+  if (r == cudaSuccess) r = cudaStreamSynchronize(st);
+  return r == cudaSuccess ? SV_OK : op_fail("attention_decode", r);
+}
+
+int sv_op_gemv_ring(const void* x, const void* w, const void* bias, const void* residual, const void* ln_w, const void* ln_b,
+                    void* y, int32_t batch, int32_t N, int32_t K, int32_t act, float ln_eps, int32_t epi, int32_t tiled,
+                    void* kcache, void* vtcache, int32_t n_head, int32_t n_kv, int32_t tcap, int32_t pos, float* amax_val,
+                    int32_t* amax_idx, int32_t amax_capacity, int32_t* ntiles_out, void* stream) {
+  if (!x || !w || !y) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: null pointer");
+  if (batch < 1 || batch > 8) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: batch %d not in [1,8]", batch);
+  if (N < 1 || K < 32 || K % 32) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: need N >= 1 and K a positive multiple of 32");
+  if (act < SV_ACT_NONE || act > SV_ACT_SILU) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: unknown act %d", act);
+  if ((ln_w == nullptr) != (ln_b == nullptr)) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: LayerNorm needs both weight and bias");
+  if (tiled != 0 && tiled != 1) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: tiled must be 0 or 1");
+  const int D = 128;
+  const int ntiles = gemv_ring_ntiles(N);
+  if (ntiles_out) *ntiles_out = ntiles;
+  if (epi == SV_GEMV_EPI_QKV) {
+    if (!kcache || !vtcache) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: QKV epilogue needs both caches");
+    if (n_kv < 1 || n_head < n_kv || n_head % n_kv || N != (n_head + 2 * n_kv) * D)
+      return fail(nullptr, SV_ERR_INVALID, "gemv_ring: QKV epilogue needs N == (n_head + 2*n_kv)*128");
+    if (tcap < 1 || pos < 0 || pos >= tcap) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: pos %d not in [0, tcap=%d)", pos, tcap);
+  } else if (epi == SV_GEMV_EPI_LMHEAD) {
+    if (!amax_val || !amax_idx) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: lm_head epilogue needs the partial buffers");
+    if (amax_capacity < ntiles) return fail(nullptr, SV_ERR_INVALID, "gemv_ring: %d partial tiles needed, capacity %d", ntiles, amax_capacity);
+  } else if (epi != SV_GEMV_EPI_PLAIN) {
+    return fail(nullptr, SV_ERR_INVALID, "gemv_ring: unknown epilogue %d", epi);
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int ncta = gemv_ring_ncta();
+  const size_t tile_bytes = tiled ? flow_tiled_bytes(N, K, ncta) : 0;
+  OpScratch s;
+  cudaError_t r = cudaMalloc(&s.p, 512 + tile_bytes);
+  if (r != cudaSuccess) return op_fail("gemv_ring alloc", r);
+  GenState* state = reinterpret_cast<GenState*>(s.p);
+  uint8_t* wt = tiled ? reinterpret_cast<uint8_t*>(s.p) + 512 : nullptr;
+  const GenState hs = op_state(epi == SV_GEMV_EPI_QKV ? pos : 0, 0);
+  r = cudaMemcpyAsync(state, &hs, sizeof(hs), cudaMemcpyHostToDevice, st);
+  if (r == cudaSuccess) r = gemv_ring_init();
+  if (r != cudaSuccess) return op_fail("gemv_ring setup", r);
+  if (tiled) launch_flow_repack((const bf16*)w, (const bf16*)bias, wt, N, K, ncta, st);
+  RingGemvLaunch g{};
+  g.X = (const bf16*)x; g.W = (const bf16*)w; g.Wt = wt; g.bias = (const bf16*)bias; g.res = (const bf16*)residual;
+  g.ln_w = (const bf16*)ln_w; g.ln_b = (const bf16*)ln_b; g.Y = (bf16*)y;
+  g.B = batch; g.N = N; g.K = K; g.act = act; g.epi = epi; g.ln_eps = ln_eps;
+  g.n_head = n_head; g.n_kv = n_kv; g.tcap = tcap; g.state = state;
+  g.kcache = (bf16*)kcache; g.vtcache = (bf16*)vtcache; g.amax_val = amax_val; g.amax_idx = amax_idx; g.pdl = false;
+  launch_gemv_ring(g, st);
+  r = cudaGetLastError();
+  if (r == cudaSuccess) r = cudaStreamSynchronize(st);
+  return r == cudaSuccess ? SV_OK : op_fail("gemv_ring", r);
+}
+
+int sv_op_select(int32_t mode, const void* logits, const uint8_t* seen, const sv_gen_params* p, int32_t batch, int32_t vocab,
+                 int32_t step, int32_t cur_len, const float* amax_val, const int32_t* amax_idx, int32_t ntiles,
+                 const void* wte, const void* wpe, int32_t h, int32_t n_positions, void* x_out, int32_t* tokens,
+                 void* stream) {
+  if (!logits || !seen || !p || !tokens) return fail(nullptr, SV_ERR_INVALID, "select: null pointer");
+  if (mode < SV_SELECT_GREEDY || mode > SV_SELECT_SAMPLE) return fail(nullptr, SV_ERR_INVALID, "select: unknown mode %d", mode);
+  if (batch < 1 || batch > 8) return fail(nullptr, SV_ERR_INVALID, "select: batch %d not in [1,8]", batch);
+  if (vocab < 1 || step < 0 || cur_len < 0) return fail(nullptr, SV_ERR_INVALID, "select: bad vocab / step / cur_len");
+  if (p->n_stop_ids < 0 || p->n_stop_ids > 8) return fail(nullptr, SV_ERR_INVALID, "select: n_stop_ids not in [0,8]");
+  if (mode == SV_SELECT_SAMPLE && !(p->temperature > 0.f && p->top_p > 0.f && p->top_p <= 1.f))
+    return fail(nullptr, SV_ERR_INVALID, "select: sampling needs temperature > 0 and top_p in (0,1]");
+  const bool fused = mode == SV_SELECT_FUSED || mode == SV_SELECT_FUSED_PARTIALS;
+  if (fused && (!wte || !x_out || h < 8 || h % 8 || (wpe && n_positions < 1)))
+    return fail(nullptr, SV_ERR_INVALID, "select: the fused kernel needs wte, x_out and h a multiple of 8");
+  if (mode == SV_SELECT_FUSED_PARTIALS && (!amax_val || !amax_idx || ntiles < 1))
+    return fail(nullptr, SV_ERR_INVALID, "select: partials mode needs amax_val, amax_idx and ntiles >= 1");
+  cudaStream_t st = (cudaStream_t)stream;
+  // scratch: GenState | params | out_ids [batch][step + 1] | next_ids [8] | seen copy [batch][vocab] | probs [batch][vocab]
+  const size_t off_par = 512, off_out = off_par + 512, out_bytes = (size_t)batch * (step + 1) * 4;
+  const size_t off_next = (off_out + out_bytes + 255) / 256 * 256, off_seen = off_next + 256;
+  const size_t off_probs = (off_seen + (size_t)batch * vocab + 255) / 256 * 256;
+  const size_t bytes = off_probs + (mode == SV_SELECT_SAMPLE ? (size_t)batch * vocab * 4 : 0);
+  OpScratch s;
+  cudaError_t r = cudaMalloc(&s.p, bytes);
+  if (r != cudaSuccess) return op_fail("select alloc", r);
+  uint8_t* base = reinterpret_cast<uint8_t*>(s.p);
+  GenState* state = reinterpret_cast<GenState*>(base);
+  GenParamsDev* par = reinterpret_cast<GenParamsDev*>(base + off_par);
+  int32_t* out_ids = reinterpret_cast<int32_t*>(base + off_out);
+  int32_t* next_ids = reinterpret_cast<int32_t*>(base + off_next);
+  uint8_t* seen_w = base + off_seen;                  // the kernels mark the chosen id: work on a copy
+  float* probs = reinterpret_cast<float*>(base + off_probs);
+  const GenState hs = op_state(cur_len, step);
+  GenParamsDev hp;
+  memset(&hp, 0, sizeof(hp));
+  hp.max_new = step + 1; hp.do_sample = p->do_sample; hp.eos_id = p->eos_token_id; hp.pad_id = p->pad_token_id;
+  hp.n_stop = p->n_stop_ids;
+  for (int i = 0; i < p->n_stop_ids; ++i) hp.stop_ids[i] = p->stop_ids[i];
+  hp.stop_row0_only = p->stop_row0_only; hp.out_stride = step + 1;
+  hp.temperature = p->temperature; hp.top_p = p->top_p; hp.rep_penalty = p->repetition_penalty; hp.seed = p->seed;
+  if ((r = cudaMemcpyAsync(state, &hs, sizeof(hs), cudaMemcpyHostToDevice, st)) != cudaSuccess ||
+      (r = cudaMemcpyAsync(par, &hp, sizeof(hp), cudaMemcpyHostToDevice, st)) != cudaSuccess ||
+      (r = cudaMemsetAsync(out_ids, 0xff, out_bytes, st)) != cudaSuccess ||
+      (r = cudaMemcpyAsync(seen_w, seen, (size_t)batch * vocab, cudaMemcpyDefault, st)) != cudaSuccess)
+    return op_fail("select setup", r);
+  if (mode == SV_SELECT_GREEDY)
+    launch_select_greedy((const bf16*)logits, vocab, batch, state, par, seen_w, next_ids, out_ids, st);
+  else if (mode == SV_SELECT_SAMPLE)
+    launch_select_sample((const bf16*)logits, vocab, batch, state, par, seen_w, next_ids, out_ids, probs, st);
+  else
+    launch_select_fused((const bf16*)logits, vocab, batch, mode == SV_SELECT_FUSED_PARTIALS ? amax_val : nullptr, amax_idx,
+                        ntiles, state, par, seen_w, next_ids, out_ids, 1, (const bf16*)wte, (const bf16*)wpe, (bf16*)x_out, h,
+                        n_positions, false, st);
+  r = cudaGetLastError();
+  if (r == cudaSuccess) r = cudaMemcpyAsync(tokens, next_ids, (size_t)batch * 4, cudaMemcpyDefault, st);
+  if (r == cudaSuccess) r = cudaStreamSynchronize(st);
+  return r == cudaSuccess ? SV_OK : op_fail("select", r);
+}
+
 }  // extern "C"

@@ -350,3 +350,65 @@ def op_attention_mqa(qkv: torch.Tensor, batch: int, seq: int, heads: int) -> tor
     out = torch.empty(batch * seq, heads * 128, dtype=torch.bfloat16, device=qkv.device)
     _lib.check(lib, lib.sv_op_attention_mqa(_p(qkv), _p(out), batch, seq, heads, _stream_ptr(qkv.device)))
     return out
+
+
+def op_attention_prefill(qkv: torch.Tensor, batch: int, seq: int, n_head: int, n_kv: int, window: int = 0) -> torch.Tensor:
+    lib = _lib.load()
+    out = torch.empty(batch * seq, n_head * 128, dtype=torch.bfloat16, device=qkv.device)
+    _lib.check(lib, lib.sv_op_attention_prefill(_p(qkv), _p(out), batch, seq, n_head, n_kv, window, _stream_ptr(qkv.device)))
+    return out
+
+
+def op_attention_decode(q: torch.Tensor, kcache: torch.Tensor, vtcache: torch.Tensor, nkeys: int, window: int = 0,
+                        impl: int = _lib.SV_ATTN_DECODE_CLUSTER, nparts: int = 0) -> torch.Tensor:
+    """q [B, n_head*128], kcache [B, n_kv, tcap, 128], vtcache [B, n_kv, 128, tcap] -> [B, n_head*128]."""
+    lib = _lib.load()
+    B, n_kv, tcap, _ = kcache.shape
+    out = torch.empty_like(q)
+    _lib.check(lib, lib.sv_op_attention_decode(impl, _p(q), _p(kcache), _p(vtcache), _p(out), B, q.shape[1] // 128, n_kv,
+                                               tcap, nkeys, window, nparts, _stream_ptr(q.device)))
+    return out
+
+
+def op_gemv_ring(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None,
+                 residual: Optional[torch.Tensor] = None, ln: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+                 act: int = 0, ln_eps: float = 1e-5, tiled: bool = False, out: Optional[torch.Tensor] = None,
+                 epi: int = _lib.SV_GEMV_EPI_PLAIN, kcache: Optional[torch.Tensor] = None,
+                 vtcache: Optional[torch.Tensor] = None, n_head: int = 0, pos: int = 0):
+    """One weight-ring decode GEMV.  `out` may alias `residual` (in-place residual).  Returns y, or for the lm_head
+    epilogue (y, amax_val [ntiles, 8], amax_idx [ntiles, 8])."""
+    lib = _lib.load()
+    B, K = x.shape
+    N = w.shape[0]
+    y = torch.empty(B, N, dtype=torch.bfloat16, device=x.device) if out is None else out
+    cap = N if epi == _lib.SV_GEMV_EPI_LMHEAD else 0
+    aval = torch.empty(cap, 8, dtype=torch.float32, device=x.device) if cap else None
+    aidx = torch.empty(cap, 8, dtype=torch.int32, device=x.device) if cap else None
+    n_kv, tcap = (kcache.shape[1], kcache.shape[2]) if kcache is not None else (0, 0)
+    ntiles = C.c_int32(0)
+    lw, lb = ln if ln is not None else (None, None)
+    _lib.check(lib, lib.sv_op_gemv_ring(_p(x), _p(w), _p(bias), _p(residual), _p(lw), _p(lb), _p(y), B, N, K, act, ln_eps, epi,
+                                        int(tiled), _p(kcache), _p(vtcache), n_head, n_kv, tcap, pos, _p(aval), _p(aidx), cap,
+                                        C.byref(ntiles), _stream_ptr(x.device)))
+    if epi == _lib.SV_GEMV_EPI_LMHEAD:
+        return y, aval[: ntiles.value], aidx[: ntiles.value]
+    return y
+
+
+def op_select(mode: int, logits: torch.Tensor, seen: torch.Tensor, params: GenerationParams, step: int = 0,
+              cur_len: int = 0, partials: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+              wte: Optional[torch.Tensor] = None, wpe: Optional[torch.Tensor] = None):
+    """One token-selection kernel on bf16 logits [B,V] and a uint8 seen bitmap [B,V].  Returns the tokens int32 [B], and for
+    the fused kernels also the embedding rows [B,h] it writes."""
+    lib = _lib.load()
+    B, V = logits.shape
+    tok = torch.empty(B, dtype=torch.int32, device=logits.device)
+    fused = mode in (_lib.SV_SELECT_FUSED, _lib.SV_SELECT_FUSED_PARTIALS)
+    h = wte.shape[1] if wte is not None else 0
+    x = torch.empty(B, h, dtype=torch.bfloat16, device=logits.device) if fused else None
+    aval, aidx = partials if partials is not None else (None, None)
+    cp = params.to_c()
+    _lib.check(lib, lib.sv_op_select(mode, _p(logits), _p(seen), C.byref(cp), B, V, step, cur_len, _p(aval), _p(aidx),
+                                     aval.shape[0] if aval is not None else 0, _p(wte), _p(wpe), h,
+                                     wpe.shape[0] if wpe is not None else 0, _p(x), _p(tok), _stream_ptr(logits.device)))
+    return (tok, x) if fused else tok
