@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SV_ABI_VERSION 5
+#define SV_ABI_VERSION 6
 #if defined(__GNUC__)
 #define SV_API __attribute__((visibility("default")))
 #else
@@ -157,6 +157,19 @@ SV_API int sv_prefill_embeds(sv_engine* e, const void* inputs_embeds, int32_t ba
 /* One teacher-forced decode step: feed ids int32 [B], append to the KV cache, return fp32 logits
  * [B,V] (optional).  The parity-test hook; also the body the generate loop replays. */
 SV_API int sv_decode_step(sv_engine* e, const int32_t* ids, float* logits, void* stream);
+/* Teacher forcing over a chunk (the scoring half of RL fine-tuning, reference StarVectorForCausalLM.forward,
+ * starvector_arch.py:161-184): append T tokens per row to the cached sequence of every row.
+ * Allowed after sv_prefill / sv_prefill_embeds / sv_expand_batch / sv_decode_step / sv_extend (not after sv_generate or
+ * sv_beam_search: SV_ERR_STATE).  ids int32 [B,T] (device), B = current batch, 1 <= T <= max_len - cur_len - 1.
+ * KV rows [cur_len, cur_len+T) are written and cur_len advances by T; the engine's last-position logits become those of
+ * the chunk's last token, so sv_decode_step / sv_extend may follow.
+ * logits (optional) float [B, keep, V]: logits of the last `keep` new positions (bf16-rounded, as HF's lm_head returns).
+ * logps  (optional) float [B, T]: logps[b][t] = log_softmax(L[b][t-1] / temperature)[ids[b][t]], in fp32, where L[b][t-1] is
+ * the bf16 logits row that predicts token t (for t = 0 the logits the engine held before the call).
+ * Runs in chunks of 4096 / B tokens (one tcgen05 GEMM of ~4096 rows per linear layer); the lm_head never writes the
+ * [B,T,V] logits for the log-probs.  Synchronises `stream`. */
+SV_API int sv_extend(sv_engine* e, const int32_t* ids, int32_t T, float* logits, int32_t keep, float* logps,
+                     float temperature, void* stream);
 /* Beam search support (SURVEY.md §8f-1): permute the image rows of the KV cache, row r <- row src_rows[r]
  * (int32 [B] on the device) for the tokens cached so far = HF `_reorder_cache` (vendored modeling_gpt_bigcode.py:1282-1291). */
 SV_API int sv_reorder_cache(sv_engine* e, const int32_t* src_rows, void* stream);
@@ -260,6 +273,11 @@ SV_API int sv_op_gemv_ring(const void* x, const void* w, const void* bias, const
                            int32_t epi, int32_t tiled, void* kcache, void* vtcache, int32_t n_head, int32_t n_kv,
                            int32_t tcap, int32_t pos, float* amax_val, int32_t* amax_idx, int32_t amax_capacity,
                            int32_t* ntiles_out, void* stream);
+/* The scoring lm_head (the hot kernel of sv_extend) on its own: x bf16 [M,K] (already final-LayerNormed), w bf16 [N,K],
+ * ids int32 [M] -> logps float [M] = log_softmax(bf16(x.w^T) / temperature)[ids] (NaN where an id is outside [0,N));
+ * logits (optional) float [M,N] = the bf16-rounded products.  Any N >= 1 (N % 8 != 0 included), K % 64 == 0. */
+SV_API int sv_op_lm_head_logps(const void* x, const void* w, const int32_t* ids, float* logps, float* logits, int32_t M,
+                               int32_t N, int32_t K, float temperature, void* stream);
 enum { SV_SELECT_GREEDY = 0, SV_SELECT_FUSED = 1, SV_SELECT_FUSED_PARTIALS = 2, SV_SELECT_SAMPLE = 3 };
 /* Token selection of one step from bf16 logits [B,V] and a seen bitmap uint8 [B,V] (host or device; not modified) at
  * generation step `step` with `cur_len` tokens in the cache -> tokens int32 [B] (host or device).  The fused kernels also

@@ -19,7 +19,7 @@ SV_LINEAR_AUTO, SV_LINEAR_ROWGROUP, SV_LINEAR_TCGEN05 = 0, 1, 2
 SV_ATTN_DECODE_CLUSTER, SV_ATTN_DECODE_SPLIT = 0, 1
 SV_GEMV_EPI_PLAIN, SV_GEMV_EPI_QKV, SV_GEMV_EPI_LMHEAD = 0, 1, 2
 SV_SELECT_GREEDY, SV_SELECT_FUSED, SV_SELECT_FUSED_PARTIALS, SV_SELECT_SAMPLE = 0, 1, 2, 3
-ABI_VERSION = 5
+ABI_VERSION = 6
 SV_ALPHA_WHITE, SV_ALPHA_DROP = 0, 1
 
 
@@ -76,6 +76,7 @@ SIGNATURES = {
     "sv_decode_step": (C.c_int, [_P, _P, _P, _P]),
     "sv_reorder_cache": (C.c_int, [_P, _P, _P]),
     "sv_expand_batch": (C.c_int, [_P, _P, C.c_int32, _P]),
+    "sv_extend": (C.c_int, [_P, _P, _I, _P, _I, _P, _F, _P]),
     "sv_beam_search": (C.c_int, [_P, C.POINTER(BeamParams), _I, _P, _P, _P]),
     "sv_beam_params_check": (C.c_int, [C.POINTER(BeamParams), _I]),
     "sv_beam_state_bytes": (C.c_int, []),
@@ -100,6 +101,7 @@ SIGNATURES = {
     "sv_op_attention_decode": (C.c_int, [_I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "sv_op_gemv_ring": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _I, _P, _P, _I, _I, _I, _I, _P, _P, _I,
                                   C.POINTER(_I), _P]),
+    "sv_op_lm_head_logps": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _F, _P]),
     "sv_op_select": (C.c_int, [_I, _P, _P, C.POINTER(GenParams), _I, _I, _I, _I, _P, _P, _I, _P, _P, _I, _I, _P, _P, _P]),
     "sv_preproc_create": (C.c_int, [C.POINTER(PreprocDesc), C.c_int, C.POINTER(_P)]),
     "sv_preproc_destroy": (None, [_P]),

@@ -173,12 +173,12 @@ void launch_attention_vit(const bf16* qkv, const bf16* vt, bf16* out, int batch,
 }
 
 // ------------------------------------------------------------------------------------------
-// Decoder (prefill): a tile = the `group` query heads of one (image, token, kv head); keys
-// [0, token] from the cache (causal).  qkv rows are [n_head*D | n_kv*D | n_kv*D].
+// Decoder (prefill / scoring chunk): a tile = the `group` query heads of one (image, token, kv head); the token sits at
+// cache position pos0 + token and takes keys [0, pos0 + token] from the cache (causal).  qkv rows are [n_head*D | n_kv*D | n_kv*D].
 template <int D>
 __global__ void __launch_bounds__(kAttnWarps * 32) attention_heads_kernel(
     const bf16* __restrict__ qkv, int ld, const bf16* __restrict__ kcache, const bf16* __restrict__ vtcache,
-    bf16* __restrict__ out, int batch, int seq, int n_head, int n_kv, int tcap, float scale_log2, int window) {
+    bf16* __restrict__ out, int batch, int seq, int n_head, int n_kv, int tcap, float scale_log2, int window, int pos0) {
   const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int tile = blockIdx.x * kAttnWarps + (threadIdx.x >> 5);
   if (tile >= batch * seq * n_kv) return;
@@ -190,8 +190,9 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attention_heads_kernel(
   float acc[D / 8][4], mrow[2], lrow[2];
   attn_init<D>(acc, mrow, lrow);
   const int64_t bk = (int64_t)b * n_kv + kvh;
-  const int key_lo = window > 0 ? max(0, tok + 1 - window) : 0;     // HF sliding window: keys in (q - window, q]
-  attn_core<D>(qa, kcache + bk * tcap * D, D, vtcache + bk * D * tcap, tcap, (key_lo / 32) * 32, tok + 1, scale_log2, acc,
+  const int qpos = pos0 + tok;
+  const int key_lo = window > 0 ? max(0, qpos + 1 - window) : 0;    // HF sliding window: keys in (q - window, q]
+  attn_core<D>(qa, kcache + bk * tcap * D, D, vtcache + bk * D * tcap, tcap, (key_lo / 32) * 32, qpos + 1, scale_log2, acc,
                mrow, lrow, lane, key_lo);
   const float inv0 = 1.0f / quad_sum(lrow[0]), inv1 = 1.0f / quad_sum(lrow[1]);
   bf16* o = out + (int64_t)bt * n_head * D + (int64_t)kvh * group * D;
@@ -206,12 +207,12 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attention_heads_kernel(
 }
 
 void launch_attention_heads(const bf16* qkv, int q_cols_total, const bf16* kcache, const bf16* vtcache, bf16* out,
-                            int batch, int seq, int n_head, int n_kv, int d, int tcap, int window, cudaStream_t st) {
+                            int batch, int seq, int n_head, int n_kv, int d, int tcap, int window, int pos0, cudaStream_t st) {
   const int tiles = batch * seq * n_kv;
   const float scale_log2 = 1.4426950408889634f / sqrtf((float)d);
   const int ld = q_cols_total;
   attention_heads_kernel<128><<<(tiles + kAttnWarps - 1) / kAttnWarps, kAttnWarps * 32, 0, st>>>(
-      qkv, ld, kcache, vtcache, out, batch, seq, n_head, n_kv, tcap, scale_log2, window);
+      qkv, ld, kcache, vtcache, out, batch, seq, n_head, n_kv, tcap, scale_log2, window, pos0);
   count_launch();
 }
 

@@ -8,6 +8,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -27,6 +28,7 @@ namespace {
 constexpr int kMaxPrompt = 64;
 constexpr int kStreamChunk = 1024;   // tokens per row handed to a streaming callback at once
 constexpr int kMaxSplit = 128;
+constexpr int kScoreRows = 4096;     // GEMM rows per sv_extend chunk (B rows x 4096 / B tokens): ~32 x 385 lm_head tiles fill 148 SMs
 
 std::string g_create_error;
 
@@ -104,6 +106,11 @@ struct sv_engine {
   int32_t *beam_tok = nullptr, *beam_run_seq = nullptr, *beam_fin_seq = nullptr;
   bf16 *kstage = nullptr, *vstage = nullptr;        // staging copy of the cache for the KV suffix moves (all layers)
   std::map<long long, GraphEntry> beam_graphs;
+  // scoring (sv_extend) workspaces for kScoreRows rows, allocated by the first sv_extend
+  bf16 *s_x = nullptr, *s_ln = nullptr, *s_qkv = nullptr, *s_attn = nullptr, *s_h = nullptr;
+  float2* s_part = nullptr;
+  float* s_tlogit = nullptr;
+  int32_t *s_tgt = nullptr, *s_lg_row = nullptr, *s_lp_idx = nullptr;
   bf16 *kcache, *vtcache;           // [layer][max_batch][n_kv][tcap][D] / [layer][max_batch][n_kv][D][tcap]
   int64_t cache_layer_stride = 0;
   GenState* state = nullptr;
@@ -439,9 +446,9 @@ int run_prefill(sv_engine* e, const bf16* prefix, int q, const int32_t* prompt_i
     launch_layernorm(e->p_x, L.ln1_w, L.ln1_b, e->p_ln, M, H, d.ln_eps, H, st);
     LIN(e->p_ln, L.attn_w, L.attn_b, nullptr, e->p_qkv, M, e->qkv_cols, H, SV_ACT_NONE, st);
     if (e->v2)   // RoPE on q and k (positions 0..T0-1), modeling_starcoder2.py:167-168
-      launch_rope(e->p_qkv, M, T0, e->qkv_cols, d.n_head + d.n_kv_head, D, e->rope_cos, e->rope_sin, nullptr, d.n_positions, st);
+      launch_rope(e->p_qkv, M, T0, e->qkv_cols, d.n_head + d.n_kv_head, D, e->rope_cos, e->rope_sin, nullptr, d.n_positions, 0, st);
     launch_kv_scatter(e->p_qkv, kc, vc, B, T0, d.n_head * D, d.n_kv_head, D, e->tcap, 0, st);
-    launch_attention_heads(e->p_qkv, e->qkv_cols, kc, vc, e->p_attn, B, T0, d.n_head, d.n_kv_head, D, e->tcap, e->window, st);
+    launch_attention_heads(e->p_qkv, e->qkv_cols, kc, vc, e->p_attn, B, T0, d.n_head, d.n_kv_head, D, e->tcap, e->window, 0, st);
     LIN(e->p_attn, L.proj_w, L.proj_b, e->p_x, e->p_x, M, H, H, SV_ACT_NONE, st);
     launch_layernorm(e->p_x, L.ln2_w, L.ln2_b, e->p_ln, M, H, d.ln_eps, H, st);
     LIN(e->p_ln, L.fc_w, L.fc_b, nullptr, e->p_h, M, d.n_inner, H, SV_ACT_GELU_TANH, st);
@@ -451,6 +458,41 @@ int run_prefill(sv_engine* e, const bf16* prefix, int q, const int32_t* prompt_i
   launch_gather_rows(e->p_x, e->d_last, B, T0, T0 - 1, H, st);
   launch_layernorm(e->d_last, e->lnf_w, e->lnf_b, e->d_ln, B, H, d.ln_eps, H, st);
   launch_linear_rowgroup(e->d_ln, e->lm_head, nullptr, nullptr, e->logits, B, d.vocab, H, SV_ACT_NONE, st);
+  return SV_OK;
+}
+
+// ---- stage: teacher forcing over a chunk (sv_extend) ------------------------------------------
+// run_prefill at a position offset: tokens ids[b][t0 .. t0 + n) of the call's [B][T] ids go to cache positions
+// pos0 .. pos0 + n (pos0 = the cache length before the call + t0).  The final LayerNorm and the lm_head with the fused log-prob
+// epilogue run on every row; the fp32 logits are stored for the rows lg_row maps (kept positions / the call's last position).
+int run_extend_chunk(sv_engine* e, const int32_t* ids, int T, int t0, int n, int pos0, int keep, float* logits_out, float* logps,
+                     float inv_temp, cudaStream_t st) {
+  const sv_model_desc& d = e->d;
+  const int B = e->cur_batch, H = d.hidden, M = B * n, D = d.head_dim;
+  launch_embed_chunk(ids + t0, T, e->wte, e->wpe, e->s_x, B, n, pos0, H, d.vocab, d.n_positions, st);
+  for (int i = 0; i < d.n_layer; ++i) {
+    const DecLayer& L = e->dec[i];
+    bf16* kc = e->kcache + e->cache_layer_stride * i;
+    bf16* vc = e->vtcache + e->cache_layer_stride * i;
+    launch_layernorm(e->s_x, L.ln1_w, L.ln1_b, e->s_ln, M, H, d.ln_eps, H, st);
+    LIN(e->s_ln, L.attn_w, L.attn_b, nullptr, e->s_qkv, M, e->qkv_cols, H, SV_ACT_NONE, st);
+    if (e->v2)
+      launch_rope(e->s_qkv, M, n, e->qkv_cols, d.n_head + d.n_kv_head, D, e->rope_cos, e->rope_sin, nullptr, d.n_positions, pos0, st);
+    launch_kv_scatter(e->s_qkv, kc, vc, B, n, d.n_head * D, d.n_kv_head, D, e->tcap, pos0, st);
+    launch_attention_heads(e->s_qkv, e->qkv_cols, kc, vc, e->s_attn, B, n, d.n_head, d.n_kv_head, D, e->tcap, e->window, pos0, st);
+    LIN(e->s_attn, L.proj_w, L.proj_b, e->s_x, e->s_x, M, H, H, SV_ACT_NONE, st);
+    launch_layernorm(e->s_x, L.ln2_w, L.ln2_b, e->s_ln, M, H, d.ln_eps, H, st);
+    LIN(e->s_ln, L.fc_w, L.fc_b, nullptr, e->s_h, M, d.n_inner, H, SV_ACT_GELU_TANH, st);
+    LIN(e->s_h, L.fc2_w, L.fc2_b, e->s_x, e->s_x, M, H, d.n_inner, SV_ACT_NONE, st);
+  }
+  // the lm_head runs where a log-prob, a kept logit or the call's last position needs it
+  const bool kept = (keep > 0 && t0 + n > T - keep) || t0 + n == T;
+  if (!logps && !kept) return SV_OK;
+  launch_layernorm(e->s_x, e->lnf_w, e->lnf_b, e->s_ln, M, H, d.ln_eps, H, st);
+  launch_score_maps(ids, T, B, n, t0, keep, d.vocab, logps != nullptr, e->s_tgt, e->s_lg_row, e->s_lp_idx, st);
+  LogpsEpilogue lp{e->s_tgt, e->s_lg_row, keep > 0 ? logits_out : e->logits_f32, e->s_part, e->s_tlogit, inv_temp};
+  cudaError_t r = launch_lm_head_logps(e->s_ln, e->lm_head, M, d.vocab, H, lp, e->s_lp_idx, logps, st);
+  if (r != cudaSuccess) return fail(e, SV_ERR_CUDA, "lm_head log-prob launch failed: %s", cudaGetErrorString(r));
   return SV_OK;
 }
 
@@ -466,7 +508,7 @@ int run_decode_layers(sv_engine* e, const int32_t* ids, int B, int nsplit, cudaS
     launch_layernorm(e->d_x, L.ln1_w, L.ln1_b, e->d_ln, B, H, d.ln_eps, H, st);
     launch_linear_rowgroup(e->d_ln, L.attn_w, L.attn_b, nullptr, e->d_qkv, B, e->qkv_cols, H, SV_ACT_NONE, st);
     if (e->v2)
-      launch_rope(e->d_qkv, B, 1, e->qkv_cols, d.n_head + d.n_kv_head, D, e->rope_cos, e->rope_sin, e->state, d.n_positions, st);
+      launch_rope(e->d_qkv, B, 1, e->qkv_cols, d.n_head + d.n_kv_head, D, e->rope_cos, e->rope_sin, e->state, d.n_positions, 0, st);
     launch_kv_append(e->d_qkv, kc, vc, e->state, B, d.n_head * D, d.n_kv_head, D, e->tcap, st);
     launch_attention_decode(e->d_qkv, e->qkv_cols, kc, vc, e->d_attn, e->attn_partial, e->state, B, d.n_head,
                             d.n_kv_head, D, e->tcap, nsplit, e->window, st);
@@ -894,6 +936,49 @@ int sv_decode_step(sv_engine* e, const int32_t* ids, float* logits, void* stream
   if (logits) launch_logits_to_float(e->logits, logits, (int64_t)e->cur_batch * e->d.vocab, st);
   SV_CK(e, cudaGetLastError());
   e->host_cur_len += 1;
+  return SV_OK;
+}
+
+int sv_extend(sv_engine* e, const int32_t* ids, int32_t T, float* logits, int32_t keep, float* logps, float temperature,
+              void* stream) {
+  if (!e || !ids) return fail(e, SV_ERR_INVALID, "null argument");
+  if (!e->prefilled)
+    return fail(e, SV_ERR_STATE, "sv_extend needs sv_prefill / sv_prefill_embeds first (a finished generation cannot be extended)");
+  const sv_model_desc& d = e->d;
+  if (T < 1 || e->host_cur_len + T + 1 > d.max_len)
+    return fail(e, SV_ERR_INVALID, "T = %d outside [1, %d] (%d tokens cached, max_len %d)", T, d.max_len - e->host_cur_len - 1,
+                e->host_cur_len, d.max_len);
+  if (keep < 0 || keep > T) return fail(e, SV_ERR_INVALID, "keep = %d outside [0, T = %d]", keep, T);
+  if (keep > 0 && !logits) return fail(e, SV_ERR_INVALID, "keep = %d needs a logits buffer", keep);
+  if (!(temperature > 0.f) || !std::isfinite(temperature)) return fail(e, SV_ERR_INVALID, "temperature must be a finite value > 0");
+  SV_CK(e, cudaSetDevice(e->device));
+  LaunchScope scope(e);
+  if (!e->s_x) {
+    const int64_t R = kScoreRows;
+    bool ok = true;
+#define SAL(ptr, n) ok = ok && (dev_alloc(e, &e->ptr, (n)) == cudaSuccess)
+    SAL(s_x, R * d.hidden); SAL(s_ln, R * d.hidden); SAL(s_qkv, R * e->qkv_cols); SAL(s_attn, R * d.hidden);
+    SAL(s_h, R * d.n_inner); SAL(s_part, R * lm_head_logps_ntiles(d.vocab)); SAL(s_tlogit, R);
+    SAL(s_tgt, R); SAL(s_lg_row, R); SAL(s_lp_idx, R);
+#undef SAL
+    if (!ok) { e->s_x = nullptr; return fail(e, SV_ERR_CUDA, "allocation of the scoring workspaces failed: %s", cudaGetErrorString(cudaGetLastError())); }
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int B = e->cur_batch, V = d.vocab, C = kScoreRows / B;
+  const float inv_temp = 1.0f / temperature;
+  if (logps) launch_row_logp(e->logits, V, B, ids, T, inv_temp, logps, T, st);    // token 0: the logits held before the call
+  for (int t0 = 0; t0 < T; t0 += C) {
+    const int r = run_extend_chunk(e, ids, T, t0, std::min(C, T - t0), e->host_cur_len + t0, keep, logits, logps, inv_temp, st);
+    if (r != SV_OK) return r;
+  }
+  // the call's last position becomes the held last-position logits (bf16-exact fp32 values -> bf16)
+  if (keep > 0) launch_float_rows_to_bf16(logits + (int64_t)(keep - 1) * V, (int64_t)keep * V, e->logits, B, V, st);
+  else launch_float_rows_to_bf16(e->logits_f32, V, e->logits, B, V, st);
+  const int32_t len = e->host_cur_len + T;
+  SV_CK(e, cudaMemcpyAsync(&e->state->cur_len, &len, sizeof(len), cudaMemcpyHostToDevice, st));   // pageable: staged synchronously
+  SV_CK(e, cudaStreamSynchronize(st));
+  SV_CK(e, cudaGetLastError());
+  e->host_cur_len = len;
   return SV_OK;
 }
 
@@ -1366,7 +1451,7 @@ int sv_op_attention_mqa(const void* qkv, void* out, int32_t batch, int32_t seq, 
   bf16* vc = kc + n;
   cudaMemsetAsync(kc, 0, 2 * n * 2, st);
   launch_kv_scatter((const bf16*)qkv, kc, vc, batch, seq, heads * D, 1, D, tcap, 0, st);
-  launch_attention_heads((const bf16*)qkv, heads * D + 2 * D, kc, vc, (bf16*)out, batch, seq, heads, 1, D, tcap, 0, st);
+  launch_attention_heads((const bf16*)qkv, heads * D + 2 * D, kc, vc, (bf16*)out, batch, seq, heads, 1, D, tcap, 0, 0, st);
   r = cudaStreamSynchronize(st);
   cudaFree(kc);
   return r == cudaSuccess ? SV_OK : op_fail("attention_mqa", r);
@@ -1385,7 +1470,7 @@ int sv_op_attention_prefill(const void* qkv, void* out, int32_t batch, int32_t s
   bf16* vc = kc + n;
   cudaMemsetAsync(kc, 0, 2 * n * 2, st);
   launch_kv_scatter((const bf16*)qkv, kc, vc, batch, seq, n_head * D, n_kv, D, tcap, 0, st);
-  launch_attention_heads((const bf16*)qkv, cols, kc, vc, (bf16*)out, batch, seq, n_head, n_kv, D, tcap, window, st);
+  launch_attention_heads((const bf16*)qkv, cols, kc, vc, (bf16*)out, batch, seq, n_head, n_kv, D, tcap, window, 0, st);
   r = cudaStreamSynchronize(st);
   cudaFree(kc);
   return r == cudaSuccess ? SV_OK : op_fail("attention_prefill", r);
@@ -1553,6 +1638,24 @@ int sv_op_select(int32_t mode, const void* logits, const uint8_t* seen, const sv
   if (r == cudaSuccess) r = cudaMemcpyAsync(tokens, next_ids, (size_t)batch * 4, cudaMemcpyDefault, st);
   if (r == cudaSuccess) r = cudaStreamSynchronize(st);
   return r == cudaSuccess ? SV_OK : op_fail("select", r);
+}
+
+int sv_op_lm_head_logps(const void* x, const void* w, const int32_t* ids, float* logps, float* logits, int32_t M, int32_t N,
+                        int32_t K, float temperature, void* stream) {
+  if (!x || !w || !ids || !logps) return fail(nullptr, SV_ERR_INVALID, "lm_head_logps: null pointer");
+  if (M < 1 || N < 1 || K < 64 || K % 64) return fail(nullptr, SV_ERR_INVALID, "lm_head_logps: need M, N >= 1 and K a positive multiple of 64");
+  if (!(temperature > 0.f) || !std::isfinite(temperature)) return fail(nullptr, SV_ERR_INVALID, "lm_head_logps: temperature must be a finite value > 0");
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t part_bytes = (size_t)M * lm_head_logps_ntiles(N) * sizeof(float2);
+  OpScratch s;
+  cudaError_t r = cudaMalloc(&s.p, part_bytes + (size_t)M * sizeof(float));
+  if (r != cudaSuccess) return op_fail("lm_head_logps alloc", r);
+  float2* part = reinterpret_cast<float2*>(s.p);
+  float* tlogit = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(s.p) + part_bytes);
+  LogpsEpilogue lp{ids, nullptr, logits, part, tlogit, 1.0f / temperature};
+  r = launch_lm_head_logps((const bf16*)x, (const bf16*)w, M, N, K, lp, nullptr, logps, st);
+  if (r == cudaSuccess) r = cudaStreamSynchronize(st);
+  return r == cudaSuccess ? SV_OK : op_fail("lm_head_logps", r);
 }
 
 }  // extern "C"

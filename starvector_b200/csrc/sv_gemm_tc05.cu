@@ -14,6 +14,12 @@
 //              row quadrants 2,3,0,1 of the tile.
 // Rows beyond M and weight rows beyond N are zero-filled by TMA (OOB fill) and masked at the store.
 // Every mbarrier wait is bounded: a protocol bug traps (CUDA error) instead of hanging the GPU.
+//
+// A second epilogue kind (EPI_LOGPS, the scoring lm_head) keeps the same producer / MMA warps and replaces the bf16 store:
+// each accumulator is rounded to bf16 (the reference lm_head's output), scaled by 1/temperature in fp32 and reduced per
+// row to a partial (max, sum exp(x - max)) over the tile's columns < N; the row's target logit is written by the one
+// tile that holds it, and the unscaled fp32 logits optionally go to a row-mapped output.  logps_merge_kernel combines the
+// partials in a fixed tile order (deterministic).
 #include <cuda.h>
 
 #include <cstdlib>
@@ -113,12 +119,14 @@ SV_DEVINL void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-template <int BN>
+enum { EPI_LINEAR = 0, EPI_LOGPS = 1 };
+
+template <int BN, int EPI>
 __global__ void __launch_bounds__(kThreads, SV_TC05_MINCTAS) linear_tc05_kernel(const __grid_constant__ CUtensorMap tmap_x,
                                                                   const __grid_constant__ CUtensorMap tmap_w,
                                                                   const bf16* __restrict__ bias,
                                                                   const bf16* __restrict__ res, bf16* __restrict__ Y,
-                                                                  int M, int N, int K, int act) {
+                                                                  int M, int N, int K, int act, const LogpsEpilogue lp) {
   using C = Cfg<BN>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -190,6 +198,51 @@ __global__ void __launch_bounds__(kThreads, SV_TC05_MINCTAS) linear_tc05_kernel(
     const int quad = warp & 3;             // TMEM lane quadrant this warp may access
     const int row = m_blk * BM + quad * 32 + lane;
     const bool has_res = res != nullptr;
+    if constexpr (EPI == EPI_LOGPS) {      // one thread = one row of the tile: no cross-thread reduction
+      const bool live = row < M;
+      const int tgt = live ? lp.tgt[row] : -1;
+      const int lrow = (live && lp.logits) ? (lp.lg_row ? lp.lg_row[row] : row) : -1;
+      float* lout = lrow >= 0 ? lp.logits + (int64_t)lrow * N : nullptr;
+      float mx = -INFINITY, sum = 0.f, tval = 0.f;
+      bool found = false;
+#pragma unroll 1
+      for (int c0 = 0; c0 < BN; c0 += 32) {
+        uint32_t r[32];
+        tmem_ld_32x32b_x32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)c0, r);   // whole warp (sync.aligned)
+        const int col0 = n_blk * BN + c0;
+        if (!live || col0 >= N) continue;
+        float lg[32];
+        float cm = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          lg[j] = bf16_round(__uint_as_float(r[j]));
+          if (col0 + j < N) cm = fmaxf(cm, lg[j] * lp.inv_temp);
+        }
+        if (cm > mx) { sum *= expf(mx - cm); mx = cm; }
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          const float xs = lg[j] * lp.inv_temp;
+          if (col0 + j < N) sum += expf(xs - mx);
+          if (col0 + j == tgt) { tval = xs; found = true; }
+        }
+        if (lout) {
+          if (col0 + 32 <= N && (N & 3) == 0) {
+#pragma unroll
+            for (int j = 0; j < 32; j += 4)
+              *reinterpret_cast<float4*>(lout + col0 + j) = make_float4(lg[j], lg[j + 1], lg[j + 2], lg[j + 3]);
+          } else {
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (col0 + j < N) lout[col0 + j] = lg[j];
+          }
+        }
+      }
+      if (live) {
+        lp.part[(int64_t)row * gridDim.x + n_blk] = make_float2(mx, sum);
+        if (found) lp.tlogit[row] = tval;
+      }
+      tcgen05_fence_before();
+    } else {
 #pragma unroll 1
     for (int c0 = 0; c0 < BN; c0 += 32) {
       uint32_t r[32];
@@ -213,6 +266,7 @@ __global__ void __launch_bounds__(kThreads, SV_TC05_MINCTAS) linear_tc05_kernel(
       }
     }
     tcgen05_fence_before();
+    }
   }
   __syncthreads();
   if (warp == 1) {
@@ -274,22 +328,52 @@ static bool cached_map(CUtensorMap* out, const void* ptr, int64_t rows, int64_t 
   return true;
 }
 
-template <int BN>
+template <int BN, int EPI = EPI_LINEAR>
 static cudaError_t launch(const bf16* x, const bf16* w, const bf16* bias, const bf16* res, bf16* y, int M, int N,
-                          int K, int act, cudaStream_t st) {
+                          int K, int act, cudaStream_t st, const LogpsEpilogue& lp = LogpsEpilogue{}) {
   CUtensorMap mx, mw;
   if (!cached_map(&mx, x, M, K, BM) || !cached_map(&mw, w, N, K, BN)) return cudaErrorInvalidValue;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(linear_tc05_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(linear_tc05_kernel<BN, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          Cfg<BN>::kSmemBytes);
     if (e != cudaSuccess) return e;
     attr_set = true;
   }
   dim3 grid((N + BN - 1) / BN, (M + BM - 1) / BM);
-  linear_tc05_kernel<BN><<<grid, kThreads, Cfg<BN>::kSmemBytes, st>>>(mx, mw, bias, res, y, M, N, K, act);
+  linear_tc05_kernel<BN, EPI><<<grid, kThreads, Cfg<BN>::kSmemBytes, st>>>(mx, mw, bias, res, y, M, N, K, act, lp);
   count_launch();
   return cudaGetLastError();
+}
+
+// One warp per row: lse = m + log(sum_i s_i * exp(m_i - m)) over the row's tile partials, lanes taking tiles lane,
+// lane + 32, ... and a fixed shuffle tree after that (the same bits on every run); logp = target logit - lse.
+SV_DEVINL void lse_combine(float& m, float& s, float m2, float s2) {
+  const float mn = fmaxf(m, m2);
+  if (mn == -INFINITY) return;
+  s = s * expf(m - mn) + s2 * expf(m2 - mn);
+  m = mn;
+}
+__global__ void logps_merge_kernel(const float2* __restrict__ part, const float* __restrict__ tlogit,
+                                   const int32_t* __restrict__ tgt, const int32_t* __restrict__ lp_idx,
+                                   float* __restrict__ logps, int M, int N, int ntiles) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (row >= M) return;
+  float m = -INFINITY, s = 0.f;
+  for (int i = lane; i < ntiles; i += 32) {
+    const float2 p = part[(int64_t)row * ntiles + i];
+    lse_combine(m, s, p.x, p.y);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float m2 = __shfl_down_sync(0xffffffffu, m, o), s2 = __shfl_down_sync(0xffffffffu, s, o);
+    lse_combine(m, s, m2, s2);
+  }
+  if (lane != 0) return;
+  const int out = lp_idx ? lp_idx[row] : row;
+  if (out < 0) return;
+  const int t = tgt[row];
+  logps[out] = (t >= 0 && t < N) ? tlogit[row] - (m + logf(s)) : __int_as_float(0x7fc00000);   // no target: NaN
 }
 
 }  // namespace tc05
@@ -310,6 +394,20 @@ cudaError_t launch_linear_tc05(const bf16* x, const bf16* w, const bf16* bias, c
   const bool wide = (N % 128 == 0) && ((int64_t)mt * ((N + 63) / 64) > (int64_t)nsm * per_sm);
   return wide ? tc05::launch<128>(x, w, bias, res, y, M, N, K, act, st)
               : tc05::launch<64>(x, w, bias, res, y, M, N, K, act, st);
+}
+
+int lm_head_logps_ntiles(int N) { return (N + 127) / 128; }
+
+cudaError_t launch_lm_head_logps(const bf16* x, const bf16* w, int M, int N, int K, const LogpsEpilogue& lp,
+                                 const int32_t* lp_idx, float* logps, cudaStream_t st) {
+  if (M < 1 || N < 1 || K < 64 || K % 64) return cudaErrorInvalidValue;
+  cudaError_t r = tc05::launch<128, tc05::EPI_LOGPS>(x, w, nullptr, nullptr, nullptr, M, N, K, /*act=*/0, st, lp);
+  if (r != cudaSuccess || !logps) return r;
+  constexpr int kRowsPerBlock = 8;
+  tc05::logps_merge_kernel<<<(M + kRowsPerBlock - 1) / kRowsPerBlock, 32 * kRowsPerBlock, 0, st>>>(
+      lp.part, lp.tlogit, lp.tgt, lp_idx, logps, M, N, lm_head_logps_ntiles(N));
+  count_launch();
+  return cudaGetLastError();
 }
 
 }  // namespace sv

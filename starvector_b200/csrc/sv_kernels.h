@@ -43,10 +43,22 @@ void launch_batchnorm_tokens(const bf16* z, const bf16* w, const bf16* b, const 
                              int batch, int q, int h, float eps, cudaStream_t st);
 void launch_embed_prefix(const bf16* visual, const int32_t* prompt_ids, const bf16* wte, const bf16* wpe, bf16* x,
                          int batch, int q, int p, int h, int vocab, cudaStream_t st);
+// teacher-forcing chunk: x[b*seq + t] = wte[ids[b*ids_ld + t]] + wpe[pos0 + t] (wpe may be nullptr)
+void launch_embed_chunk(const int32_t* ids, int ids_ld, const bf16* wte, const bf16* wpe, bf16* x, int batch, int seq, int pos0,
+                        int h, int vocab, int n_positions, cudaStream_t st);
+// per-row maps of one scoring chunk (rows b*seq + t, t0 + t = position in the call's T tokens), see sv_extend
+void launch_score_maps(const int32_t* ids, int T, int batch, int seq, int t0, int keep, int vocab, bool want_logps,
+                       int32_t* tgt, int32_t* lg_row, int32_t* lp_idx, cudaStream_t st);
+// logps[b*lp_ld] = log_softmax(logits[b] / T)[ids[b*ids_ld]] over bf16 rows [batch][vocab] (one block per row)
+void launch_row_logp(const bf16* logits, int vocab, int batch, const int32_t* ids, int ids_ld, float inv_temp, float* logps,
+                     int lp_ld, cudaStream_t st);
+// dst bf16 [batch][n] = src fp32 rows (row b at src + b * src_ld), values already bf16-exact
+void launch_float_rows_to_bf16(const float* src, int64_t src_ld, bf16* dst, int batch, int n, cudaStream_t st);
 void launch_embed_tokens(const int32_t* ids, const bf16* wte, const bf16* wpe, const GenState* state, bf16* x,
                          int batch, int h, int vocab, int n_positions, cudaStream_t st);
+// cache positions pos0 .. pos0 + seq - 1 of every row
 void launch_kv_scatter(const bf16* qkv, bf16* kcache, bf16* vtcache, int batch, int seq, int q_cols, int n_kv, int d,
-                       int tcap, int max_batch_unused, cudaStream_t st);
+                       int tcap, int pos0, cudaStream_t st);
 void launch_kv_append(const bf16* qkv, bf16* kcache, bf16* vtcache, const GenState* state, int batch, int q_cols,
                       int n_kv, int d, int tcap, cudaStream_t st);
 void launch_kv_gather(const bf16* ksrc, const bf16* vsrc, bf16* kdst, bf16* vdst, const int32_t* idx, int rows, int n_kv,
@@ -70,20 +82,36 @@ bool tc05_supported(int M, int N, int K);
 // returns cudaSuccess or the error of tensor-map creation / launch
 cudaError_t launch_linear_tc05(const bf16* x, const bf16* w, const bf16* bias, const bf16* res, bf16* y, int M, int N,
                                int K, int act, cudaStream_t st);
+// Scoring lm_head: logits = bf16(x[M,K] . w[N,K]^T) (any N >= 1, K % 64 == 0) reduced on the fly to log-probs of one target
+// per row, logp = logits[tgt] / T - logsumexp(logits / T), without writing the logits (unless `logits` is given).
+struct LogpsEpilogue {
+  const int32_t* tgt;     // [M] target column of each row; < 0: no target
+  const int32_t* lg_row;  // [M] output row of the fp32 logits (< 0: not stored); nullptr = identity
+  float* logits;          // fp32 [.., N] bf16-rounded unscaled logits, or nullptr
+  float2* part;           // [M][lm_head_logps_ntiles(N)] per-tile (max, sum exp(x - max)) of the scaled row
+  float* tlogit;          // [M] scaled target logit
+  float inv_temp;
+};
+int lm_head_logps_ntiles(int N);
+// GEMM + partials, then (logps != nullptr) the merge: logps[lp_idx ? lp_idx[r] : r] = logp of row r (lp_idx[r] < 0: skipped;
+// a row without target gets NaN)
+cudaError_t launch_lm_head_logps(const bf16* x, const bf16* w, int M, int N, int K, const LogpsEpilogue& lp,
+                                 const int32_t* lp_idx, float* logps, cudaStream_t st);
 
 // ---- sv_attention.cu
 void launch_attention_vit(const bf16* qkv, const bf16* vt, bf16* out, int batch, int seq, int heads, int seq_pad,
                           cudaStream_t st);
-// causal attention of `seq` new tokens per row against the cache (prefill: cache already holds them)
+// causal attention of `seq` new tokens per row against the cache (which already holds them): token t of a row sits at
+// cache position pos0 + t and attends to keys [0 | pos0 + t + 1 - window, pos0 + t]
 void launch_attention_heads(const bf16* qkv, int q_cols_total, const bf16* kcache, const bf16* vtcache, bf16* out,
-                            int batch, int seq, int n_head, int n_kv, int d, int tcap, int window, cudaStream_t st);
+                            int batch, int seq, int n_head, int n_kv, int d, int tcap, int window, int pos0, cudaStream_t st);
 void launch_attention_decode(const bf16* qkv, int q_cols_total, const bf16* kcache, const bf16* vtcache, bf16* out,
                              float* partial, const GenState* state, int batch, int n_head, int n_kv, int d, int tcap,
                              int nsplit, int window, cudaStream_t st);
 // RoPE in place on the q and k parts of packed qkv rows [rows][qkv_cols] (StarCoder2, rotate_half convention);
 // cos/sin tables are bf16 [max_pos][D/2]; position of row r = pos0 + (r % seq) or state->cur_len when state != nullptr.
 void launch_rope(bf16* qkv, int rows, int seq, int qkv_cols, int n_rot_heads, int d, const bf16* cos_t, const bf16* sin_t,
-                 const GenState* state, int max_pos, cudaStream_t st);
+                 const GenState* state, int max_pos, int pos0, cudaStream_t st);
 void launch_rope_append(bf16* qkv, int batch, int qkv_cols, int n_head, int n_kv, int d, const bf16* cos_t,
                         const bf16* sin_t, bf16* kcache, bf16* vtcache, const GenState* state, int tcap, int max_pos,
                         bool pdl, cudaStream_t st);

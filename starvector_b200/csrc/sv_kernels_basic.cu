@@ -266,6 +266,103 @@ void launch_embed_prefix(const bf16* visual, const int32_t* prompt_ids, const bf
   count_launch();
 }
 
+__global__ void embed_chunk_kernel(const int32_t* __restrict__ ids, int ids_ld, const bf16* __restrict__ wte,
+                                   const bf16* __restrict__ wpe, bf16* __restrict__ x, int seq, int pos0, int h, int vocab,
+                                   int n_positions) {
+  const int b = blockIdx.x / seq, t = blockIdx.x % seq;
+  int id = ids[(int64_t)b * ids_ld + t];
+  id = id < 0 ? 0 : (id >= vocab ? vocab - 1 : id);
+  const int pos = min(pos0 + t, n_positions - 1);
+  const bf16* src = wte + (int64_t)id * h;
+  const bf16* pe = wpe ? wpe + (int64_t)pos * h : nullptr;
+  for (int c = threadIdx.x * 8; c < h; c += blockDim.x * 8) {
+    float a[8], d[8];
+    unpack8(ldg_cached(src + c), a);
+    if (pe) {
+      unpack8(ldg_cached(pe + c), d);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) a[j] += d[j];
+    }
+    *reinterpret_cast<uint4*>(x + (int64_t)blockIdx.x * h + c) = pack8(a);
+  }
+}
+void launch_embed_chunk(const int32_t* ids, int ids_ld, const bf16* wte, const bf16* wpe, bf16* x, int batch, int seq, int pos0,
+                        int h, int vocab, int n_positions, cudaStream_t st) {
+  embed_chunk_kernel<<<batch * seq, 128, 0, st>>>(ids, ids_ld, wte, wpe, x, seq, pos0, h, vocab, n_positions);
+  count_launch();
+}
+
+// Row r = b*seq + t of a scoring chunk holds call position t0 + t; its logits predict token t0 + t + 1 of the row.
+//   tgt    : that token's id (clamped as the embedding clamps), -1 past the end
+//   lp_idx : where its log-prob goes in logps [B][T], -1 past the end or when no log-probs are wanted
+//   lg_row : output row of its fp32 logits: the last `keep` positions go to [B][keep]; with keep == 0 only the call's last
+//            position is stored, to row b of a [B][V] staging buffer (it becomes the engine's held last-position logits)
+__global__ void score_maps_kernel(const int32_t* __restrict__ ids, int T, int rows, int seq, int t0, int keep, int vocab,
+                                  int want_logps, int32_t* __restrict__ tgt, int32_t* __restrict__ lg_row,
+                                  int32_t* __restrict__ lp_idx) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= rows) return;
+  const int b = r / seq, t = t0 + r % seq;
+  int id = -1;
+  if (t + 1 < T) {
+    id = ids[(int64_t)b * T + t + 1];
+    id = id < 0 ? 0 : (id >= vocab ? vocab - 1 : id);
+  }
+  tgt[r] = id;
+  lp_idx[r] = (want_logps && t + 1 < T) ? b * T + t + 1 : -1;
+  lg_row[r] = keep > 0 ? (t >= T - keep ? b * keep + t - (T - keep) : -1) : (t == T - 1 ? b : -1);
+}
+void launch_score_maps(const int32_t* ids, int T, int batch, int seq, int t0, int keep, int vocab, bool want_logps,
+                       int32_t* tgt, int32_t* lg_row, int32_t* lp_idx, cudaStream_t st) {
+  const int rows = batch * seq;
+  score_maps_kernel<<<(rows + 255) / 256, 256, 0, st>>>(ids, T, rows, seq, t0, keep, vocab, want_logps ? 1 : 0, tgt, lg_row,
+                                                        lp_idx);
+  count_launch();
+}
+
+// log_softmax(bf16 row / T)[id] with the lm_head epilogue's arithmetic: x = bf16 value * (1/T) in fp32, fp32 max and sum.
+__global__ void row_logp_kernel(const bf16* __restrict__ logits, int vocab, const int32_t* __restrict__ ids, int ids_ld,
+                                float inv_temp, float* __restrict__ logps, int lp_ld) {
+  __shared__ float red[32];
+  const int b = blockIdx.x, nw = blockDim.x >> 5, w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const bf16* row = logits + (int64_t)b * vocab;
+  float m = -INFINITY;
+  for (int i = threadIdx.x; i < vocab; i += blockDim.x) m = fmaxf(m, __bfloat162float(row[i]) * inv_temp);
+  m = warp_max(m);
+  if (lane == 0) red[w] = m;
+  __syncthreads();
+  m = -INFINITY;
+  for (int i = 0; i < nw; ++i) m = fmaxf(m, red[i]);
+  __syncthreads();
+  float s = 0.f;
+  for (int i = threadIdx.x; i < vocab; i += blockDim.x) s += expf(__bfloat162float(row[i]) * inv_temp - m);
+  s = warp_sum(s);
+  if (lane == 0) red[w] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    s = 0.f;
+    for (int i = 0; i < nw; ++i) s += red[i];
+    int id = ids[(int64_t)b * ids_ld];
+    id = id < 0 ? 0 : (id >= vocab ? vocab - 1 : id);
+    logps[(int64_t)b * lp_ld] = __bfloat162float(row[id]) * inv_temp - (m + logf(s));
+  }
+}
+void launch_row_logp(const bf16* logits, int vocab, int batch, const int32_t* ids, int ids_ld, float inv_temp, float* logps,
+                     int lp_ld, cudaStream_t st) {
+  row_logp_kernel<<<batch, 256, 0, st>>>(logits, vocab, ids, ids_ld, inv_temp, logps, lp_ld);
+  count_launch();
+}
+
+__global__ void float_rows_to_bf16_kernel(const float* __restrict__ src, int64_t src_ld, bf16* __restrict__ dst, int n) {
+  const int b = blockIdx.y;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    dst[(int64_t)b * n + i] = __float2bfloat16_rn(src[b * src_ld + i]);
+}
+void launch_float_rows_to_bf16(const float* src, int64_t src_ld, bf16* dst, int batch, int n, cudaStream_t st) {
+  float_rows_to_bf16_kernel<<<dim3((n + 255) / 256 < 64 ? (n + 255) / 256 : 64, batch), 256, 0, st>>>(src, src_ld, dst, n);
+  count_launch();
+}
+
 __global__ void embed_tokens_kernel(const int32_t* __restrict__ ids, const bf16* __restrict__ wte,
                                     const bf16* __restrict__ wpe, const GenState* __restrict__ state,
                                     bf16* __restrict__ x, int h, int vocab, int n_positions) {
@@ -298,9 +395,9 @@ void launch_embed_tokens(const int32_t* ids, const bf16* wte, const bf16* wpe, c
 // (so the P.V tensor-core operand is a contiguous 16-byte load per lane; see sv_attention.cu).
 // The reference re-allocates and copies the whole cache every step (torch.cat, SURVEY.md K15).
 __global__ void kv_write_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ kcache, bf16* __restrict__ vtcache,
-                                const GenState* __restrict__ state, int seq, int q_cols, int n_kv, int d, int tcap) {
+                                const GenState* __restrict__ state, int seq, int q_cols, int n_kv, int d, int tcap, int pos0) {
   const int b = blockIdx.y, ts = blockIdx.x;
-  const int t = state ? state->cur_len + ts : ts;
+  const int t = (state ? state->cur_len : pos0) + ts;
   if (t >= tcap) return;
   const int cols = q_cols + 2 * n_kv * d;
   const bf16* row = qkv + ((int64_t)b * seq + ts) * cols;
@@ -311,13 +408,13 @@ __global__ void kv_write_kernel(const bf16* __restrict__ qkv, bf16* __restrict__
   }
 }
 void launch_kv_scatter(const bf16* qkv, bf16* kcache, bf16* vtcache, int batch, int seq, int q_cols, int n_kv, int d,
-                       int tcap, int, cudaStream_t st) {
-  kv_write_kernel<<<dim3(seq, batch), 128, 0, st>>>(qkv, kcache, vtcache, nullptr, seq, q_cols, n_kv, d, tcap);
+                       int tcap, int pos0, cudaStream_t st) {
+  kv_write_kernel<<<dim3(seq, batch), 128, 0, st>>>(qkv, kcache, vtcache, nullptr, seq, q_cols, n_kv, d, tcap, pos0);
   count_launch();
 }
 void launch_kv_append(const bf16* qkv, bf16* kcache, bf16* vtcache, const GenState* state, int batch, int q_cols,
                       int n_kv, int d, int tcap, cudaStream_t st) {
-  kv_write_kernel<<<dim3(1, batch), 128, 0, st>>>(qkv, kcache, vtcache, state, 1, q_cols, n_kv, d, tcap);
+  kv_write_kernel<<<dim3(1, batch), 128, 0, st>>>(qkv, kcache, vtcache, state, 1, q_cols, n_kv, d, tcap, 0);
   count_launch();
 }
 
@@ -585,9 +682,9 @@ void launch_rope_table(bf16* cos_t, bf16* sin_t, int max_pos, int d, float theta
 }
 __global__ void rope_kernel(bf16* __restrict__ qkv, int seq, int qkv_cols, int n_rot_heads, int d,
                             const bf16* __restrict__ cos_t, const bf16* __restrict__ sin_t,
-                            const GenState* __restrict__ state, int max_pos) {
+                            const GenState* __restrict__ state, int max_pos, int pos0) {
   const int row = blockIdx.x, half = d >> 1;
-  int pos = state ? state->cur_len : (row % seq);
+  int pos = state ? state->cur_len : pos0 + (row % seq);
   pos = pos >= max_pos ? max_pos - 1 : pos;
   bf16* base = qkv + (int64_t)row * qkv_cols;
   for (int i = threadIdx.x; i < n_rot_heads * half; i += blockDim.x) {
@@ -649,8 +746,8 @@ void launch_rope_append(bf16* qkv, int batch, int qkv_cols, int n_head, int n_kv
 }
 
 void launch_rope(bf16* qkv, int rows, int seq, int qkv_cols, int n_rot_heads, int d, const bf16* cos_t, const bf16* sin_t,
-                 const GenState* state, int max_pos, cudaStream_t st) {
-  rope_kernel<<<rows, 256, 0, st>>>(qkv, seq, qkv_cols, n_rot_heads, d, cos_t, sin_t, state, max_pos);
+                 const GenState* state, int max_pos, int pos0, cudaStream_t st) {
+  rope_kernel<<<rows, 256, 0, st>>>(qkv, seq, qkv_cols, n_rot_heads, d, cos_t, sin_t, state, max_pos, pos0);
   count_launch();
 }
 

@@ -198,6 +198,24 @@ class Engine:
                                               _stream_ptr(self.device)))
         return logits
 
+    def extend(self, ids: torch.Tensor, keep_logits: int = 0, logps: bool = True,
+               temperature: float = 1.0) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+        """`sv_extend`: teacher-force ids `[B, T]` after the cached sequence of every row (after a prefill, `expand_batch`,
+        `decode_step` or another `extend`).  Returns `(logits, logps)`: fp32 logits `[B, keep_logits, V]` of the last
+        `keep_logits` new positions (None when 0) and fp32 `[B, T]` log-probs `log_softmax(L / temperature)[ids]`, where
+        position t is scored by the logits that predict it (t = 0: the logits held before the call); None unless `logps`."""
+        t = self._dev(ids, torch.int32)
+        if t.dim() != 2 or t.shape[0] != self._batch:
+            raise ValueError(f"ids must be [B, T] with B = {self._batch} rows of the current batch")
+        B, T = t.shape
+        keep = int(keep_logits)
+        lg = torch.empty(B, keep, self.dims.vocab, dtype=torch.float32, device=self.device) if keep > 0 else None
+        lp = torch.empty(B, T, dtype=torch.float32, device=self.device) if logps else None
+        with self._lock:
+            self._ck(self._lib.sv_extend(self._h, C.c_void_p(t.data_ptr()), T, _p(lg), keep, _p(lp), float(temperature),
+                                         _stream_ptr(self.device)))
+        return lg, lp
+
     def reorder_cache(self, src_rows: torch.Tensor) -> None:
         """KV-cache row permutation for beam search: row r <- row src_rows[r]."""
         idx = self._dev(src_rows, torch.int32).reshape(-1)
@@ -393,6 +411,21 @@ def op_gemv_ring(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] 
     if epi == _lib.SV_GEMV_EPI_LMHEAD:
         return y, aval[: ntiles.value], aidx[: ntiles.value]
     return y
+
+
+def op_lm_head_logps(x: torch.Tensor, w: torch.Tensor, ids: torch.Tensor, temperature: float = 1.0,
+                     return_logits: bool = False):
+    """The scoring lm_head: x bf16 [M,K], w bf16 [N,K], ids int [M] -> fp32 logps [M] = log_softmax(bf16(x.w^T) / T)[ids]
+    (NaN where an id is outside [0,N)); with `return_logits` also the fp32 [M,N] bf16-rounded logits."""
+    lib = _lib.load()
+    M, K = x.shape
+    N = w.shape[0]
+    tid = ids.to(device=x.device, dtype=torch.int32).contiguous()
+    lp = torch.empty(M, dtype=torch.float32, device=x.device)
+    lg = torch.empty(M, N, dtype=torch.float32, device=x.device) if return_logits else None
+    _lib.check(lib, lib.sv_op_lm_head_logps(_p(x), _p(w), _p(tid), _p(lp), _p(lg), M, N, K, float(temperature),
+                                            _stream_ptr(x.device)))
+    return (lp, lg) if return_logits else lp
 
 
 def op_select(mode: int, logits: torch.Tensor, seen: torch.Tensor, params: GenerationParams, step: int = 0,

@@ -361,15 +361,10 @@ class StarVectorForCausalLM:
         write_checkpoint(path, self.config, state_dict)
 
     # -- scoring (starvector_arch.py:161-184) ------------------------------------------------
-    @torch.no_grad()
-    def forward(self, vision_embeds: torch.Tensor, input_ids: torch.Tensor, num_generations: int = 1,
-                attention_mask: Optional[torch.Tensor] = None, num_logits_to_keep: int = 0):
-        """Logits of `num_generations` completions per image over a shared visual prefix, as the reference's
-        `StarVectorForCausalLM.forward`: `inputs_embeds = cat([vision_embeds.repeat(G, 1, 1), wte(input_ids)], 1)` -> decoder
-        -> `lm_head` on the last `num_logits_to_keep` positions (all completion positions when 0).  Here the prefix is
-        prefilled ONCE per image and its KV rows replicated (`sv_expand_batch`, rows r % b as `.repeat` orders them); the
-        completion is teacher-forced through `sv_decode_step`.  Returns an object with `.logits` fp32 `[b*G, n_keep, V]`
-        and `.loss = None`.  `attention_mask` may only mask a right-padded tail (what GRPO completions carry)."""
+    def _scoring_rows(self, vision_embeds: torch.Tensor, input_ids: torch.Tensor, num_generations: int,
+                      attention_mask: Optional[torch.Tensor]):
+        """Shared argument rules of `forward` and `per_token_logps`: `b * G` completion rows in `.repeat` order, and only a
+        right-padded tail may be masked.  Prefills the prefix ONCE per image and replicates its KV rows (row r <- r % b)."""
         eng = self.model.engine
         b, G = vision_embeds.shape[0], int(num_generations)
         ids = input_ids.to(eng.device)
@@ -383,19 +378,50 @@ class StarVectorForCausalLM:
             tail = m[:, m.shape[1] - T:] if m.shape[1] >= T else m
             if not bool(torch.all(m[:, : m.shape[1] - T])) or bool(torch.any(tail[:, 1:] & ~tail[:, :-1])):
                 raise NotImplementedError("only right-padded completions (mask = ones then zeros) are supported")
+        return eng, b, G, ids, T
+
+    @torch.no_grad()
+    def forward(self, vision_embeds: torch.Tensor, input_ids: torch.Tensor, num_generations: int = 1,
+                attention_mask: Optional[torch.Tensor] = None, num_logits_to_keep: int = 0):
+        """Logits of `num_generations` completions per image over a shared visual prefix, as the reference's
+        `StarVectorForCausalLM.forward`: `inputs_embeds = cat([vision_embeds.repeat(G, 1, 1), wte(input_ids)], 1)` -> decoder
+        -> `lm_head` on the last `num_logits_to_keep` positions (all completion positions when 0; T + 1 adds the prefix's
+        last position, TRL's `logits_to_keep + 1`).  Here the prefix is prefilled ONCE per image and its KV rows replicated
+        (`sv_expand_batch`, rows r % b as `.repeat` orders them); the completion is teacher-forced through `sv_decode_step`.
+        Returns an object with `.logits` fp32 `[b*G, n_keep, V]` and `.loss = None`.  `attention_mask` may only mask a
+        right-padded tail (what GRPO completions carry).  Log-probs for RL: `per_token_logps` computes them without the logits."""
+        eng, b, G, ids, T = self._scoring_rows(vision_embeds, input_ids, num_generations, attention_mask)
         n_keep = T if int(num_logits_to_keep) <= 0 else int(num_logits_to_keep)
-        if n_keep > T:
-            raise NotImplementedError("num_logits_to_keep beyond the completion (prefix positions) is not built")
+        if n_keep > T + 1:
+            raise NotImplementedError("num_logits_to_keep beyond the completion and the prefix's last position is not built")
+        lead = eng.prefill_embeds(vision_embeds.to(eng.device, torch.bfloat16), return_logits=n_keep == T + 1)
+        if G > 1:
+            eng.expand_batch([r % b for r in range(b * G)])
+        n_body = min(n_keep, T)
+        out = torch.empty(b * G, n_body, eng.dims.vocab, dtype=torch.float32, device=eng.device)
+        for t in range(T):
+            keep = t >= T - n_body
+            lg = eng.decode_step(ids[:, t], return_logits=keep)
+            if keep:
+                out[:, t - (T - n_body)] = lg
+        if n_keep == T + 1:
+            out = torch.cat([lead[[r % b for r in range(b * G)]].unsqueeze(1), out], dim=1)
+        return _ScoreOutput(loss=None, logits=out)
+
+    @torch.no_grad()
+    def per_token_logps(self, vision_embeds: torch.Tensor, input_ids: torch.Tensor, num_generations: int = 1,
+                        attention_mask: Optional[torch.Tensor] = None, temperature: float = 1.0) -> torch.Tensor:
+        """What a GRPO trainer computes from `forward(..., num_logits_to_keep=T + 1).logits`: fp32 `[b*G, T]` with
+        `[r, t] = log_softmax(logits[r, t] / temperature)[input_ids[r, t]]`, where logits[r, t] is the row predicting
+        completion token t (t = 0: the prefix's last position).  Rows and mask rules as `forward`; the caller applies the
+        mask to the result.  One prefill per image, then the completions in chunks through `sv_extend`, whose lm_head reduces
+        its tiles to log-probs on the fly: the `[b*G, T, V]` logits are never written."""
+        eng, b, G, ids, T = self._scoring_rows(vision_embeds, input_ids, num_generations, attention_mask)
         eng.prefill_embeds(vision_embeds.to(eng.device, torch.bfloat16))
         if G > 1:
             eng.expand_batch([r % b for r in range(b * G)])
-        out = torch.empty(b * G, n_keep, eng.dims.vocab, dtype=torch.float32, device=eng.device)
-        for t in range(T):
-            keep = t >= T - n_keep
-            lg = eng.decode_step(ids[:, t], return_logits=keep)
-            if keep:
-                out[:, t - (T - n_keep)] = lg
-        return _ScoreOutput(loss=None, logits=out)
+        _, lp = eng.extend(ids, logps=True, temperature=temperature)
+        return lp
 
     __call__ = forward
 
